@@ -8,8 +8,10 @@ by the NCCL all-reduce of the per-object hit counts.  Weak scaling: every rank e
 its own 65,536 hypotheses; `value` is the whole-job rate.
 
   python bench.py [--gpus N --steps K --warmup W]        our arm (one process per GPU)
+  python bench.py [...] --dump-outputs DIR               also write the per-pose outputs of the last timed
+                                                         step as DIR/<name>.npy (see dump_outputs)
   python bench.py --impl reference [...]                 CPU arm: the UNMODIFIED reference
-        (baseline/_ref, P6D_REFERENCE or /root/reference: ADDLoss.eval_metrics in batches of 16 on
+        (baseline/_ref or P6D_REFERENCE: ADDLoss.eval_metrics in batches of 16 on
         all host cores) when it is reachable, else the oracle port of its algorithm; same metric,
         bounded sample per step
 
@@ -41,6 +43,7 @@ import numpy as np
 REPO = os.path.dirname(os.path.abspath(__file__))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 N_POINTS = 2048
 POSES_PER_GPU = 65536
@@ -69,7 +72,12 @@ def parse():
     ap.add_argument("--sweep-per-block", type=int, default=1_000_000, help="hypotheses per (object, variant) block")
     ap.add_argument("--sweep-points", default="500,2048", help="mesh sizes of the sweep record")
     ap.add_argument("--sweep-check", type=int, default=256, help="poses per block checked against the oracle")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed on rank 0 to DIR/<name>.npy (float32 / float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def config_dict(args, extra=None):
@@ -201,7 +209,7 @@ def real_reference():
         from oracle import torch_eager as E
         root = E.find_reference()
         if root is None:
-            return None, "no reference checkout (P6D_REFERENCE, baseline/_ref, /root/reference)"
+            return None, "no reference checkout (P6D_REFERENCE, baseline/_ref)"
         W = importlib.import_module("6d-pose-estimation_b200.workloads")
         pts, dia = W.config2_meshes(N_POINTS)
         return root, E.reference_criterion(root, pts, dia)
@@ -585,6 +593,37 @@ def sweep_record(pkg, dev, rank, world, n_points, n_per_block, check_total, barr
                                      "bits and decisions vs oracle/pose_oracle.c"}}
 
 
+# ------------------------------------------------------------------------- outputs
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, last, acc, counts=None):
+    """What a caller of MeshTable.evaluate received from the last timed step, one DIR/<name>.npy per array:
+    per-pose add, adds (metres), hit, valid and the per-object accumulators obj_hits, obj_valid, obj_add_sum,
+    obj_adds_sum (at N > 1 also the all-reduced obj_hits_all_ranks, obj_valid_all_ranks).  Integers are
+    stored as float64, hit / valid as float32.  The inputs are seeded, so two builds run with the same
+    arguments can be compared file by file.  When the per-pose arrays would exceed 64 MB, a fixed seeded
+    sample of poses is written instead, with its row numbers in pose_index."""
+    import torch
+    add, adds, hit, valid, _ = last
+    per_pose = {"add": add.float(), "adds": adds.float(), "hit": hit.float(), "valid": valid.float()}
+    per_object = {"obj_hits": acc[0], "obj_valid": acc[1], "obj_add_sum": acc[2], "obj_adds_sum": acc[3]}
+    if counts is not None:
+        per_object.update(obj_hits_all_ranks=counts[0], obj_valid_all_ranks=counts[1])
+    arrays = {k: v.double().cpu().numpy() for k, v in per_object.items()}
+    n = add.shape[0]
+    room = DUMP_BYTES - sum(a.nbytes for a in arrays.values()) - 4096       # 4 KB for the .npy headers
+    if 16 * n > room:                  # 4 float32 per pose; a sample also stores its float64 row numbers
+        idx = np.sort(np.random.default_rng(0).choice(n, room // 24, replace=False))
+        arrays["pose_index"] = idx.astype(np.float64)
+        sel = torch.from_numpy(idx).to(add.device)
+        per_pose = {k: v[sel] for k, v in per_pose.items()}
+    arrays.update({k: v.cpu().numpy() for k, v in per_pose.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------- GPU arm
 def run_b200(args):
     import torch
@@ -618,12 +657,13 @@ def run_b200(args):
     counts = torch.zeros(2, table.n_slots, dtype=torch.int64, device=dev)
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     launches = 0
+    last = None
 
     def step():
-        nonlocal launches
+        nonlocal launches, last
         for a in acc:
             a.zero_()
-        table.evaluate(*d_in, want_adds=True, order=order, acc=acc)
+        last = table.evaluate(*d_in, want_adds=True, order=order, acc=acc)
         launches += 1
         if world > 1:
             counts[0].copy_(acc[0]); counts[1].copy_(acc[1])
@@ -667,6 +707,8 @@ def run_b200(args):
     # result sanity on the numbers just computed (accuracy is counts / totals, integer-exact)
     hits = int(acc[0].sum().item()); valid = int(acc[1].sum().item())
     assert valid == B, (valid, B)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, acc, counts if world > 1 else None)
 
     # ---------------- end-to-end: host buffers in, host results out, through the C ABI
     def e2e(bufs):

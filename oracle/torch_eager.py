@@ -13,7 +13,7 @@ calls, in its order, on the local CPU, with no knowledge of any rounding rule.
     quat_to_mat              models/add_loss.py:203-215
     resolve_borderline       decisions for poses the kernels flag as within 4 ulp of the threshold
     find_reference / load_reference   the unmodified reference, when reachable
-                             (P6D_REFERENCE, baseline/_ref, /root/reference)
+                             (P6D_REFERENCE, baseline/_ref)
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs use this
 module.
@@ -121,8 +121,8 @@ def resolve_borderline(points: dict, diameters: dict):
 
 # --------------------------------------------------------------------------- the real reference
 def find_reference() -> str | None:
-    """Directory of the unmodified reference if this machine has one."""
-    for cand in (os.environ.get("P6D_REFERENCE"), os.path.join(_REPO, "baseline", "_ref"), "/root/reference"):
+    """Directory of the unmodified reference if this machine has one (P6D_REFERENCE, or baseline/_ref)."""
+    for cand in (os.environ.get("P6D_REFERENCE"), os.path.join(_REPO, "baseline", "_ref")):
         if cand and os.path.isfile(os.path.join(cand, "models", "add_loss.py")):
             return cand
     return None
