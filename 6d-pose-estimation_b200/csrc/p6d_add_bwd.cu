@@ -3,8 +3,9 @@
 // The reference gets this from autograd through matmul / norm / min / mean
 // (models/add_loss.py:101-150), materialising [n,N,N,3] for symmetric objects (1.6 GB at
 // n=32, N=2048).  Here: one CTA per pose, the gt cloud in shared memory, each thread owns
-// pred points, finds the nearest gt point (first index on ties, like torch.min) with a
-// value+index scan, and accumulates dL/dt (3) and dL/dR (9) in float64; thread 0 applies
+// pred points, finds the nearest gt point (the first index whose ROOTED distance is minimal,
+// like torch.norm(...).min: equal roots of different squares tie) with a value+index scan, and
+// accumulates dL/dt (3) and dL/dR (9) in float64; thread 0 applies
 // the quaternion Jacobian of _quat_to_mat (add_loss.py:203-215, no normalisation).
 //   loss = (1/count) * sum_b mean_i d_bi ,  d = |p_i - g_i| (ADD) or min_j |p_i - g_j| (ADD-S)
 //   dL/dp_i = scale * (p_i - g*) / d   (0 where d == 0, PyTorch's norm sub-gradient)
@@ -82,13 +83,26 @@ __global__ void __launch_bounds__(BWD_T) add_backward_kernel(BwdArgs a, int nmax
             xform_point(s.xform_bmm, m0, m1, m2, Rp, tp, px, py, pz);
             int js = i;
             if (s.symmetric) {
-                float best = __int_as_float(0x7f800000);
+                float best = __int_as_float(0x7f800000), prev = best;  // prev: the minimum before best
                 js = 0;
                 bool nan_seen = false;
                 for (int j = 0; j < n; ++j) {
                     const float sv = sq3(__fsub_rn(px, gx[j]), __fsub_rn(py, gy[j]), __fsub_rn(pz, gz[j]));
                     if (sv != sv && !nan_seen) { nan_seen = true; js = j; best = sv; }
-                    if (!nan_seen && sv < best) { best = sv; js = j; }
+                    if (!nan_seen && sv < best) { prev = best; best = sv; js = j; }
+                }
+                // torch.min runs on the ROOTED distances: an earlier point whose square is larger but
+                // whose sqrt equals sqrt(best) is the nearest one.  Its square is >= prev (the running
+                // minimum before js), so there is none unless sqrt(prev) == sqrt(best); only then
+                // (rare) rescan [0, js).
+                if (!nan_seen && js > 0 && __fsqrt_rn(prev) == __fsqrt_rn(best)) {
+                    const float r = __fsqrt_rn(best);
+                    for (int j = 0; j < js; ++j) {
+                        if (__fsqrt_rn(sq3(__fsub_rn(px, gx[j]), __fsub_rn(py, gy[j]), __fsub_rn(pz, gz[j]))) == r) {
+                            js = j;
+                            break;
+                        }
+                    }
                 }
             }
             const float dx = __fsub_rn(px, gx[js]), dy = __fsub_rn(py, gy[js]), dz = __fsub_rn(pz, gz[js]);

@@ -107,6 +107,14 @@ __device__ __forceinline__ RowOut loss_row(const float4 a4, const float* pt_row,
         float dn, sn, cd, cs;
         if (FAST) {
             const float sd = sumsq4(d), ss = sumsq4(s);
+            // Two decisions of the exact row are discontinuous in u and v: the sign of dot (it negates
+            // the gradient) and dn == 0 (zero gradient instead of a unit vector along rounding noise).
+            // A FAST u or v differs from the exact one by <= ~10 ulp per component (RSQ 2 ulp, sums and
+            // products), so the FAST dot is within ~28 * 2^-24 < 2^-19 of the exact dot, and a FAST
+            // |d|^2 is below (20 * 2^-24)^2 < 2^-39 where the exact d is 0.  Near either edge (margins
+            // >= 8x) the row is recomputed exactly; uniformly random pairs land there with probability ~1e-5.
+            if (fabsf(dot) < 0x1p-16f || sd < 0x1p-30f)
+                return loss_row<false>(a4, pt_row, c4, gt_row, B, wr, wt, mode, grad_q_row, grad_t_row);
             const float rd = sd > 0.0f ? rsqrtf(sd) : 0.0f, rs = ss > 0.0f ? rsqrtf(ss) : 0.0f;
             dn = sd * rd;
             sn = ss * rs;
@@ -161,7 +169,8 @@ __device__ __forceinline__ RowOut loss_row(const float4 a4, const float* pt_row,
         for (int k = 0; k < 4; ++k) gp[k] = scale * fmaf(-u[k], proj, gu[k]);
         *reinterpret_cast<float4*>(grad_q_row) = g4;
     }
-    const float tscale = (float)((double)wt / (3.0 * (double)B));
+    // ATen's mean backward divides in float32 by float32(numel), which is inexact once 3B > 2^24
+    const float tscale = __fdiv_rn(wt, (float)(3 * B));
 #pragma unroll
     for (int k = 0; k < 3; ++k) {
         const float df = __fsub_rn(pt_row[k], gt_row[k]);

@@ -361,12 +361,19 @@ P6O_API int p6o_add_backward(const float* mesh_xyz, const int32_t* offsets, cons
             p6o_xform_point(mesh + 3 * i, Rp, pt + 3 * b, P6O_BMM(n), p);
             int64_t js = i;
             if (symmetric[oid]) {
-                float best = INFINITY;
+                /* torch.norm(...).min(dim=2): the first j with the smallest ROOTED distance.  Two
+                 * different squares can have the same sqrtf; the earlier point wins then.  best_r
+                 * is always sqrtf(best), so the root is only taken when the square improves. */
+                float best = INFINITY, best_r = INFINITY;
                 js = 0;
                 for (int64_t j = 0; j < n; ++j) {
                     const float sv = p6o_sq3(p[0] - g[3 * j], p[1] - g[3 * j + 1], p[2] - g[3 * j + 2]);
                     if (sv != sv) { js = j; break; }
-                    if (sv < best) { best = sv; js = j; }
+                    if (sv < best) {
+                        best = sv;
+                        const float r = sqrtf(sv);
+                        if (r < best_r) { best_r = r; js = j; }
+                    }
                 }
             }
             const float d3[3] = {p[0] - g[3 * js], p[1] - g[3 * js + 1], p[2] - g[3 * js + 2]};
@@ -483,8 +490,9 @@ P6O_API int p6o_pose_loss(const float* pq, const float* pt, const float* gq, con
             const float df = pt[3 * b + k] - gt[3 * b + k];
             absd[3 * b + k] = fabsf(df);
             if (grad_t) {
-                const double sg = (df > 0) - (df < 0);
-                grad_t[3 * b + k] = (float)((double)trans_weight * sg / (3.0 * (double)B));
+                /* ATen's mean backward: float32(weight) / float32(numel), then times sign */
+                const float sg = (float)((df > 0) - (df < 0));
+                grad_t[3 * b + k] = sg * (trans_weight / (float)(3 * B));
             }
         }
     }

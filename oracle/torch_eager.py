@@ -11,6 +11,9 @@ calls, in its order, on the local CPU, with no knowledge of any rounding rule.
     eval_pose / eval_poses   models/add_loss.py:168-195 (loop body of ADDLoss.eval_metrics)
     forward_value            models/add_loss.py:101-150 (ADDLoss.forward)
     quat_to_mat              models/add_loss.py:203-215
+    add_loss_grad, pose_loss_grad, geometric_loss_grad, pinhole_translation
+                             the gradients of ADDLoss.forward, PoseLoss.forward and the RGB-Geometric
+                             step under autograd, in float32 and in float64 (tests/test_gradients.py)
     resolve_borderline       decisions for poses the kernels flag as within 4 ulp of the threshold
     find_reference / load_reference   the unmodified reference, when reachable
                              (P6D_REFERENCE, baseline/_ref)
@@ -105,6 +108,147 @@ def forward_value(points: dict, pq, pt, gq, gt, obj) -> np.float32:
         total = total + per.sum()
         count += len(idx)
     return np.float32(0.0) if count == 0 else np.float32((total / count).item())
+
+
+# --------------------------------------------------------------------------- autograd references
+# Each gradient reference runs in two forms.  float32 (decisions=None) is the reference's own op
+# sequence under autograd: it rounds like the reference, so it takes the reference's discrete decisions,
+# and it returns them.  float64 (dtype=torch.float64, decisions=<those>) repeats the computation on the
+# same inputs with every discrete decision taken from the float32 run -- nearest-point indices, the
+# dot < 0 flip, the L1 branch, the 1e-12 clamp, zero distances and sign(0) -- because float64 takes
+# other branches on degenerate rows (an antipodal prediction scaled by 3 has a gradient of exactly 0 in
+# float32, not in float64).  Within those decisions the float64 form is the exact gradient up to 1e-15.
+def _const(a, dtype, shape):
+    return torch.from_numpy(np.array(a)).reshape(shape).to(dtype)
+
+
+def _leaf(a, dtype, shape):
+    return _const(a, dtype, shape).requires_grad_(True)
+
+
+def add_loss_grad(points: dict, pq, pt, gq, gt, obj, grad_out=1.0, dtype=torch.float32, decisions=None):
+    """(grad_q [B,4], grad_t [B,3], decisions) of ADDLoss.forward (models/add_loss.py:101-150) under
+    autograd.  The clouds are transformed per object group with the reference's batched matmul; the
+    nearest gt point of a symmetric object is found per sample with the reference's own
+    ``torch.norm(...).min(dim=2)`` (no [n,N,N,3] graph for all n at once), and the gradient flows through
+    the chosen points, which is what min's backward does.  decisions: per sample, the chosen gt index of
+    every pred point and the mask of zero distances."""
+    B = np.asarray(obj).size
+    a, b = _leaf(pq, dtype, (B, 4)), _leaf(pt, dtype, (B, 3))
+    gqt, gtt = _const(gq, dtype, (B, 4)), _const(gt, dtype, (B, 3))
+    objs = np.asarray(obj, np.int64).ravel()
+    meshes = {int(k): _const(v, dtype, (-1, 3)) for k, v in points.items()}
+    Rp, Rg = quat_to_mat(a), quat_to_mat(gqt)
+    groups: dict[int, list[int]] = {}
+    for i, o in enumerate(objs):
+        if int(o) in meshes:
+            groups.setdefault(int(o), []).append(i)
+    count = sum(len(v) for v in groups.values())
+    out_dec = {}
+    total = None
+    for oid, idx in groups.items():
+        idx_t = torch.tensor(idx, dtype=torch.long)
+        m = meshes[oid].unsqueeze(0)
+        cg = torch.matmul(m, Rg[idx_t].transpose(-1, -2)) + gtt[idx_t].unsqueeze(1)
+        cp = torch.matmul(m, Rp[idx_t].transpose(-1, -2)) + b[idx_t].unsqueeze(1)
+        for k, s in enumerate(idx):
+            if decisions is None:
+                if oid in SYMMETRIC:
+                    with torch.no_grad():
+                        near = torch.norm(cp[k].unsqueeze(1) - cg[k].unsqueeze(0), dim=2).min(dim=1)[1]
+                else:
+                    near = torch.arange(m.shape[1])
+                diff = cp[k] - cg[k][near]
+                d = torch.norm(diff, dim=1)
+                out_dec[s] = (near, (d == 0).detach())
+            else:
+                near, zero = decisions[s]
+                diff = (cp[k] - cg[k][near]) * (~zero).to(dtype).unsqueeze(1)
+                d = torch.norm(diff, dim=1)
+            term = d.mean()
+            total = term if total is None else total + term
+    if total is None:
+        z = np.zeros((B, 4), np.float64 if dtype == torch.float64 else np.float32)
+        return z, z[:, :3].copy(), out_dec
+    loss = total / count
+    loss.backward(torch.tensor(grad_out, dtype=dtype))
+    ga = a.grad if a.grad is not None else torch.zeros_like(a)
+    gb = b.grad if b.grad is not None else torch.zeros_like(b)
+    return ga.numpy(), gb.numpy(), (out_dec if decisions is None else decisions)
+
+
+def pose_loss_grad(pq, pt, gq, gt, rot_weight=1.0, trans_weight=1.0, mode="geodesic", grad_out=1.0,
+                   dtype=torch.float32, decisions=None):
+    """(loss, grad_q [B,4], grad_t [B,3], decisions) of PoseLoss.forward (models/pose_loss.py:19-61) under
+    autograd: F.normalize, where(dot < 0), 2*atan2(|q1-q2|, |q1+q2|) or the torch.min of the two L1 sums,
+    F.l1_loss, the weights.  Anything but 'geodesic' selects the L1 distance, as in the reference."""
+    import torch.nn.functional as F
+    B = np.asarray(pq).size // 4
+    a, b = _leaf(pq, dtype, (B, 4)), _leaf(pt, dtype, (B, 3))
+    c, g = _const(gq, dtype, (B, 4)), _const(gt, dtype, (B, 3))
+    if decisions is None:
+        q1, q2 = F.normalize(a, dim=1), F.normalize(c, dim=1)
+        dec = {"clamp": (torch.norm(a.detach(), dim=1) < 1e-12)}
+        if mode == "geodesic":
+            dot = torch.sum(q1 * q2, dim=1, keepdim=True)
+            q2 = torch.where(dot < 0, -q2, q2)
+            dn, sn = torch.norm(q1 - q2, dim=1), torch.norm(q1 + q2, dim=1)
+            rot = (2 * torch.atan2(dn, sn)).mean()
+            dec.update(flip=(dot < 0).detach(), dn0=(dn == 0).detach(), sn0=(sn == 0).detach())
+        else:
+            dp, dm = torch.sum(torch.abs(q1 - q2), dim=1), torch.sum(torch.abs(q1 + q2), dim=1)
+            rot = torch.min(dp, dm).mean()
+            dec.update(wp=torch.where(dp < dm, 1.0, torch.where(dp == dm, 0.5, 0.0)).detach(),
+                       ap0=(q1 - q2 == 0).detach(), am0=(q1 + q2 == 0).detach())
+        dec["t0"] = (b - g == 0).detach()
+        trans = F.l1_loss(b, g)
+    else:
+        dec = decisions
+        keep = lambda x, zero: x * (~zero).to(dtype)
+        na = torch.where(dec["clamp"], torch.full((B,), 1e-12, dtype=dtype), torch.norm(a, dim=1))
+        q1 = a / na.unsqueeze(1)
+        q2 = c / torch.norm(c, dim=1).clamp_min(1e-12).unsqueeze(1)
+        if mode == "geodesic":
+            q2 = torch.where(dec["flip"], -q2, q2)
+            dn = torch.norm(keep(q1 - q2, dec["dn0"].unsqueeze(1)), dim=1)
+            sn = torch.norm(keep(q1 + q2, dec["sn0"].unsqueeze(1)), dim=1)
+            rot = (2 * torch.atan2(dn, sn)).mean()
+        else:
+            wp = dec["wp"].to(dtype)
+            dp = torch.sum(torch.abs(keep(q1 - q2, dec["ap0"])), dim=1)
+            dm = torch.sum(torch.abs(keep(q1 + q2, dec["am0"])), dim=1)
+            rot = (wp * dp + (1 - wp) * dm).mean()
+        trans = torch.abs(keep(b - g, dec["t0"])).mean()
+    loss = rot_weight * rot + trans_weight * trans
+    loss.backward(torch.tensor(grad_out, dtype=dtype))
+    return loss.item(), a.grad.numpy(), b.grad.numpy(), dec
+
+
+def pinhole_translation(z, uv, K):
+    """PoseNetRGBGeometric._compute_pinhole_translation (models/pose_net_rgb_geometric.py:93-109) on
+    tensors: [(u - cx) * z / fx, (v - cy) * z / fy, z], K [3,3] or [B,3,3]; differentiable in z."""
+    K = K.reshape(-1, 3, 3)
+    fx, fy, cx, cy = K[:, 0, 0:1], K[:, 1, 1:2], K[:, 0, 2:3], K[:, 1, 2:3]
+    z = z.reshape(-1, 1)
+    return torch.cat([(uv[:, 0:1] - cx) * z / fx, (uv[:, 1:2] - cy) * z / fy, z], dim=1)
+
+
+def geometric_loss_grad(pq, z, uv, K, gq, gt, rot_weight=1.0, trans_weight=1.0, mode="geodesic", grad_out=1.0,
+                        dtype=torch.float32, decisions=None):
+    """(loss, grad_q [B,4], grad_z [B,1], decisions): PoseLoss on the pinhole translation, autograd through
+    both (the RGB-Geometric training step, train_rgb_geometric.py:104-108)."""
+    B = np.asarray(pq).size // 4
+    zz = _leaf(z, dtype, (B, 1))
+    tr = pinhole_translation(zz, _const(uv, dtype, (B, 2)), _const(K, dtype, (-1, 3, 3)))
+    t32 = tr.detach().to(torch.float32).numpy() if dtype == torch.float32 else None
+    if decisions is None:
+        loss, gq_, gt_, dec = pose_loss_grad(pq, t32, gq, gt, rot_weight, trans_weight, mode, grad_out)
+    else:
+        dec = decisions
+        loss, gq_, gt_, _ = pose_loss_grad(pq, tr.detach().numpy(), gq, gt, rot_weight, trans_weight, mode,
+                                           grad_out, torch.float64, dec)
+    tr.backward(torch.from_numpy(gt_).to(dtype))
+    return loss, gq_, zz.grad.numpy(), dec
 
 
 def resolve_borderline(points: dict, diameters: dict):
