@@ -30,7 +30,8 @@ P6D_VERSION = 4
 EXPORTS = (
     "p6d_version", "p6d_last_error", "p6d_device_info", "p6d_mesh_table_create",
     "p6d_mesh_table_destroy", "p6d_adds_max_points", "p6d_adds_schedule", "p6d_adds_schedule_state",
-    "p6d_adds_selfcheck", "p6d_selftest_sqrt2", "p6d_add_eval", "p6d_add_eval_pruned", "p6d_mesh_table_set_pruning", "p6d_add_eval_host",
+    "p6d_adds_selfcheck", "p6d_selftest_sqrt2", "p6d_add_eval", "p6d_add_eval_pruned", "p6d_mesh_table_set_pruning", "p6d_add_eval_streamed",
+    "p6d_mesh_table_set_large_meshes", "p6d_add_eval_host",
     "p6d_add_forward_workspace_bytes", "p6d_add_forward", "p6d_add_backward",
     "p6d_quat_to_mat", "p6d_pose_loss_workspace_bytes", "p6d_pose_loss_fwd_bwd",
     "p6d_pose_loss_pinhole_fwd_bwd", "p6d_pinhole_fwd", "p6d_pinhole_bwd", "p6d_depth_backproject",
@@ -85,6 +86,8 @@ def lib() -> C.CDLL:
     L.p6d_add_eval.argtypes = [vp, vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, C.POINTER(Accumulators), vp]
     L.p6d_add_eval_pruned.argtypes = L.p6d_add_eval.argtypes
     L.p6d_mesh_table_set_pruning.argtypes = [vp, i32]
+    L.p6d_add_eval_streamed.argtypes = L.p6d_add_eval.argtypes
+    L.p6d_mesh_table_set_large_meshes.argtypes = [vp, i32]
     L.p6d_add_eval_host.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                     C.POINTER(i32)]
     L.p6d_add_forward_workspace_bytes.argtypes = [vp, i64]
@@ -226,31 +229,42 @@ class MeshTable:
         check(lib().p6d_mesh_table_set_pruning(self.handle, 1 if enable else 0))
         return self
 
+    def set_large_meshes(self, enable=True):
+        """Opt in to (or out of) the streamed ADD / ADD-S kernel for this table: same bits as the resident
+        kernels, taken only when the largest mesh is beyond their shared-memory limit (up to 32,768 points);
+        see include/p6d.h."""
+        check(lib().p6d_mesh_table_set_large_meshes(self.handle, 1 if enable else 0))
+        return self
+
     # -- device-buffer evaluation ---------------------------------------------------
-    def evaluate_packed(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False):
+    def evaluate_packed(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False):
         """Launch the evaluation kernels on the current stream and return the ONE buffer behind the
         per-pose outputs: add f32 [B] | adds f32 [B] | hit u8 [B] | valid u8 [B] | borderline u8 [B]
         (adds is left unwritten when want_adds is False).  All inputs must already be contiguous CUDA
         tensors on this table's device.  No views are created: at the reference's batch sizes every
-        torch op is 2-3 us of a ~100 us call."""
+        torch op is 2-3 us of a ~100 us call.  prune / streamed: always the exact-pruned (ADD-S only) or the
+        streamed kernel (p6d_add_eval_pruned / p6d_add_eval_streamed) instead of the table's choice."""
         B = obj.shape[0]
         out = torch.empty(11 * B + 16, dtype=torch.uint8, device=self.device)
         base = out.data_ptr()
         acc_struct = None
         if acc is not None:
             acc_struct = Accumulators(*(ptr(a) for a in acc))
-        entry = lib().p6d_add_eval_pruned if (prune and want_adds) else lib().p6d_add_eval
+        if streamed:
+            entry = lib().p6d_add_eval_streamed
+        else:
+            entry = lib().p6d_add_eval_pruned if (prune and want_adds) else lib().p6d_add_eval
         check(entry(self.handle, pq.data_ptr(), pt.data_ptr(), gq.data_ptr(), gt.data_ptr(), obj.data_ptr(),
                     ptr(order), B, base, (base + 4 * B) if want_adds else None, base + 8 * B, base + 9 * B,
                     base + 10 * B, C.byref(acc_struct) if acc_struct is not None else None,
                     stream_ptr(self.device)))
         return out
 
-    def evaluate(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False):
+    def evaluate(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False):
         """evaluate_packed + views: returns (add, adds, hit, valid, packed) device tensors (adds is
         None when want_adds is False)."""
         B = obj.shape[0]
-        out = self.evaluate_packed(pq, pt, gq, gt, obj, want_adds, order, acc, prune)
+        out = self.evaluate_packed(pq, pt, gq, gt, obj, want_adds, order, acc, prune, streamed)
         add = out[: 4 * B].view(torch.float32)
         adds = out[4 * B: 8 * B].view(torch.float32)
         return add, (adds if want_adds else None), out[8 * B: 9 * B], out[9 * B: 10 * B], out

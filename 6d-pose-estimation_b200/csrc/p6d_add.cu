@@ -599,6 +599,10 @@ static int configure_variant(const p6d_mesh_table* t, int vi, size_t smem, int* 
     return P6D_OK;
 }
 
+// p6d_adds_streamed.cu: the opt-in kernel for meshes beyond shared memory (p6d_mesh_table_set_large_meshes)
+bool large_meshes_enabled(const p6d_mesh_table* t);
+int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st);
+
 void fill_eval_args(const p6d_mesh_table* t, EvalArgs& a) {
     a.soa = t->d_soa;
     a.pair = t->d_pair;
@@ -628,6 +632,17 @@ int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, c
         if (used) {
             if (launches) ++*launches;
             return P6D_OK;
+        }
+        // opt-in (p6d_mesh_table_set_large_meshes): the streamed kernel, only where the resident one cannot run
+        if (large_meshes_enabled(t)) {
+            int limit = 0;
+            const int rc2 = max_optin_smem(t->device, &limit);
+            if (rc2) return rc2;
+            if (adds_smem_bytes(t->max_count) + 256 > static_cast<size_t>(limit)) {
+                const int rc3 = launch_eval_streamed(t, args, true, st);
+                if (rc3 == P6D_OK && launches) ++*launches;
+                return rc3;
+            }
         }
     }
     int vi = force_variant;
@@ -801,6 +816,8 @@ int p6d_adds_max_points(int device, int* max_points) {
 // block structure of the opt-in pruned ADD-S kernel (p6d_adds_pruned.cu)
 void p6d_internal_build_pruned(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets);
 void p6d_internal_release_pruned(const p6d_mesh_table* t);
+// per-table switch of the streamed kernel (p6d_adds_streamed.cu)
+void p6d_internal_release_streamed(const p6d_mesh_table* t);
 
 int p6d_mesh_table_create(const float* xyz, const int32_t* offsets, const int32_t* counts,
                           const double* diameters, const uint8_t* symmetric, int n_slots, int device,
@@ -885,6 +902,7 @@ int p6d_mesh_table_destroy(p6d_mesh_table* t) {
     if (!t) return P6D_OK;
     DeviceGuard guard(t->device);
     p6d_internal_release_pruned(t);
+    p6d_internal_release_streamed(t);
     if (t->stream) cudaStreamDestroy(t->stream);
     if (t->d_stage) cudaFree(t->d_stage);
     if (t->h_pinned) cudaFreeHost(t->h_pinned);

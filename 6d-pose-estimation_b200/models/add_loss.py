@@ -76,12 +76,16 @@ class ADDLoss(nn.Module):
         self._table = None
         self._table_key = None
         self._table_pruning = False
+        self._table_large = False
         # optional callable(indices, pred_r, pred_t, gt_r, gt_t, obj_ids) -> 0/1 per index, consulted by
         # eval_metrics for decisions flagged `borderline`; None (default): the kernel's decision stands
         self.borderline_resolver = None
         # opt-in: exact block pruning in the ADD-S kernel (same bits; pays for meshes of >= 128 points, the
         # all-pairs kernel is kept below that) -- not part of the reference surface, default off
         self.exact_pruning = False
+        # opt-in: meshes beyond shared memory (up to 32,768 points) through the streamed kernel in eval_metrics /
+        # eval_poses (same bits; forward keeps its limit) -- not part of the reference surface, default off
+        self.large_meshes = False
         self._load_models(model_dir)
 
     # ------------------------------------------------------------------ loading
@@ -144,9 +148,13 @@ class ADDLoss(nn.Module):
             self._table = _core().MeshTable(self.points, self.diameters, SYMMETRIC_OBJECT_IDS, device)
             self._table_key = key
             self._table_pruning = False
+            self._table_large = False
         if bool(self.exact_pruning) != self._table_pruning:
             self._table.set_pruning(bool(self.exact_pruning))
             self._table_pruning = bool(self.exact_pruning)
+        if bool(self.large_meshes) != self._table_large:
+            self._table.set_large_meshes(bool(self.large_meshes))
+            self._table_large = bool(self.large_meshes)
         return self._table
 
     def _prepare(self, pred_r, pred_t, gt_r, gt_t, obj_ids, sort=True):

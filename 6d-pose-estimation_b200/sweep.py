@@ -114,11 +114,13 @@ class PoseEvaluator:
     """Device-resident ADD / ADD-S / ADD-0.1d evaluation over large hypothesis sets."""
 
     def __init__(self, points: dict, diameters: dict, device, symmetric_ids=SYMMETRIC_OBJECT_IDS,
-                 n_rows: int = 1, exact_pruning: bool = False):
+                 n_rows: int = 1, exact_pruning: bool = False, large_meshes: bool = False):
         self.device = core.require_cuda(device)
         self.table = core.MeshTable(points, diameters, symmetric_ids, self.device)
         if exact_pruning:       # opt-in: same bits from the pruned ADD-S kernel where the table qualifies
             self.table.set_pruning(True)
+        if large_meshes:        # opt-in: meshes beyond shared memory (up to 32,768 points) through the streamed kernel
+            self.table.set_large_meshes(True)
         self.acc = Accumulators(n_rows, self.table.n_slots, self.device)
         self.launches = 0
 
@@ -188,7 +190,7 @@ def variant_translation(variant: str, block: dict, K):
 def evaluate_sweep(points: dict, diameters: dict, device, n_per_block: int, variants=VARIANTS, chunk: int = 1 << 20,
                    seed: int = 5000, rank: int = 0, world: int = 1, group=None, K=None, check_n: int = 0,
                    rot_sigma: float = 0.05, trans_sigma: float = 0.005, evaluator: "PoseEvaluator | None" = None,
-                   exact_pruning: bool = False):
+                   exact_pruning: bool = False, large_meshes: bool = False):
     """compare_all_models-style sweep (reference scripts/visualization/compare_all_models.py:65-104 at the
     scale of BASELINE config 5): for every (object, variant) block, `n_per_block` seeded hypotheses, the
     hypothesis axis of each block sliced across `world` ranks (`shard_range`).  The whole sweep of this
@@ -198,7 +200,8 @@ def evaluate_sweep(points: dict, diameters: dict, device, n_per_block: int, vari
     `check` holds the first `check_n` hypotheses of every block of this rank's slice exactly as they
     were evaluated (inputs and outputs, host arrays) for an independent re-evaluation, or None."""
     dev = core.require_cuda(device)
-    ev = evaluator or PoseEvaluator(points, diameters, dev, n_rows=len(variants), exact_pruning=exact_pruning)
+    ev = evaluator or PoseEvaluator(points, diameters, dev, n_rows=len(variants), exact_pruning=exact_pruning,
+                                    large_meshes=large_meshes)
     if K is None:
         from .utils.camera import DEFAULT_K
         K = DEFAULT_K

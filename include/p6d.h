@@ -142,6 +142,25 @@ int p6d_add_eval_pruned(const p6d_mesh_table* table, const float* pq, const floa
                         float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                         const p6d_accumulators* acc, void* stream);
 
+/* OPT-IN: the same outputs, bit for bit, for meshes larger than shared memory.  The resident kernels stage the whole
+ * mesh in shared memory and answer P6D_ETOOBIG beyond p6d_adds_max_points (ADD-S) or ~16,700 points (ADD only,
+ * adds = NULL); this kernel streams the gt cloud through shared memory in tiles of 1,024 points (TMA bulk copies,
+ * transformed by the gt pose per tile) and splits every pose into blocks of pred points, so it takes meshes of up to
+ * 32,768 points.  Above that, torch's CPU Tensor.mean() sums a row on several threads and the reference's own result
+ * depends on the caller's thread count: such tables answer P6D_ETOOBIG.  It allocates a workspace of 8 bytes per point
+ * and pose (at most 64 MB; larger batches run in chunks) stream-ordered on `stream`; no host synchronisation.
+ *   p6d_add_eval_streamed            always this kernel, for any mesh of 1 to 32,768 points; adds = NULL gives the
+ *                                    ADD-only outputs (symmetric ids then decide on ADD)
+ *   p6d_mesh_table_set_large_meshes  per-table switch (default off): p6d_add_eval, p6d_add_eval_host and p6d_sweep_run
+ *                                    then take this kernel for a table whose largest mesh is beyond the resident
+ *                                    kernel's limit, and the resident kernels otherwise (the loss form
+ *                                    p6d_add_forward and p6d_add_backward keep their limit). */
+int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable);
+int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                          const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
+                          float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                          const p6d_accumulators* acc, void* stream);
+
 /* Same computation with HOST buffers: stages inputs to the device, runs the kernels,
  * copies results back and synchronises (the end-to-end path of bench.py).  acc_* are
  * host arrays [n_slots] that receive (not accumulate) the per-object totals; nullable.
