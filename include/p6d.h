@@ -181,7 +181,13 @@ int p6d_add_eval_host(p6d_mesh_table* table, const float* pq, const float* pt, c
  *   workspace: device buffer of p6d_add_forward_workspace_bytes(table, B) bytes, 16-byte aligned
  * Bit-exact against the reference for meshes of up to 44 points (ATen's naive bmm kernel) and
  * from 45 points on (MKL, fused chain), except group sizes for which MKL's batched sgemm takes
- * another path (observed: exactly 2 samples of a 97...106- or 200-point mesh): 1e-5 there.
+ * another path: 1e-5 there.  tests/test_loss_form.py measures where, on the machine it runs on,
+ * over n = 1...3,000 points x g = 1...257 samples per group (24 x 17 points).  Measured: on an
+ * 8-thread x86 CPU (torch 2.11.0, MKL) exactly 2 samples of a 97- or a 200-point mesh, ADD-S
+ * only.  A point outside g = 2, n = 97...106 or 200 fails the test by name.
+ * Groups of more than 32,768 samples are summed in the order of torch's CPU sum on ONE thread.
+ * With more threads torch splits such a sum, so the reference's own value then depends on the
+ * caller's thread count (measured: within 1e-5).  Such batches are accepted, not refused.
  * ------------------------------------------------------------------------------------- */
 int64_t p6d_add_forward_workspace_bytes(const p6d_mesh_table* table, int64_t B);
 int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
