@@ -15,6 +15,7 @@
 //
 // Arithmetic is the reference's, rounding for rounding (DESIGN.md "Arithmetic"); the
 // final means use aten_sum_warp so the float32 results equal the CPU reference's bits.
+#include <algorithm>
 #include <atomic>
 #include <cmath>
 #include <cstdarg>
@@ -47,13 +48,12 @@ int cuda_fail(cudaError_t e, const char* what) {
 }
 
 // ------------------------------------------------------------------ kernel (b): ADD-S
-constexpr float SENTINEL = 1.0e18f;  // padded gt coordinate: (p - 1e18)^2 * 3 < FLT_MAX, never the min
 constexpr int ADDS_MAX_U = 2;        // largest quad-unroll of any variant (sizes the gt padding)
 
 // dynamic shared memory layout (floats), for a table whose largest mesh has Nmax points:
 //   mesh  [3 * Npmax]            staged by TMA; x | y | z, each Np long
 //   gt    [3 * Ngmax]            gt cloud as quads {x0..x3 | y0..y3 | z0..z3} (48 B per 4 points, one
-//                                pointer + immediate offsets in the scan), padded with SENTINEL to 4*S*U
+//                                pointer + immediate offsets in the scan), padded with GT_SENTINEL to 4*S*U
 //   dadd  [Nmax], dadds [Nmax]   per-point distances for the ordered means
 //   mbar  8 bytes
 __host__ __device__ inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -61,18 +61,6 @@ __host__ __device__ inline int adds_ngmax(int nmax) { return round_up(nmax, 4) +
 static inline size_t adds_smem_bytes(int nmax) {
     const int np = round_up(nmax, 4);
     return sizeof(float) * (3 * (size_t)np + 3 * (size_t)adds_ngmax(nmax) + 2 * (size_t)np) + 16;
-}
-
-__device__ __forceinline__ void pair_tile(float px, float py, float pz, float2 gx, float2 gy, float2 gz,
-                                          float& m) {
-    // two (pred, gt) pairs: 3 FADD2 + FMUL2 + 2 FFMA2 + FMNMX3.NAN
-    const float2 dx = sub2(make_float2(px, px), gx);
-    const float2 dy = sub2(make_float2(py, py), gy);
-    const float2 dz = sub2(make_float2(pz, pz), gz);
-    float2 s = mul2(dx, dx);
-    s = fma2(dy, dy, s);
-    s = fma2(dz, dz, s);
-    m = min3_nan(m, s.x, s.y);
 }
 
 // U quads starting at p (quad stride `step` float4s) against K register-resident pred points
@@ -96,16 +84,6 @@ __device__ __forceinline__ void scan_quads(const float4* __restrict__ p, int ste
                       make_float2(Z[u].z, Z[u].w), m[k]);
         }
     }
-}
-
-// two pairs of one tile without the minimum: the squared distances go to `s`
-__device__ __forceinline__ float2 pair_sq(float px, float py, float pz, float2 gx, float2 gy, float2 gz) {
-    const float2 dx = sub2(make_float2(px, px), gx);
-    const float2 dy = sub2(make_float2(py, py), gy);
-    const float2 dz = sub2(make_float2(pz, pz), gz);
-    float2 s = mul2(dx, dx);
-    s = fma2(dy, dy, s);
-    return fma2(dz, dz, s);
 }
 
 // Software-pipelined form of the unit-stride scan (one quad per trip): the minima of trip t are
@@ -330,9 +308,9 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
                     s_dadd[i] = __fsqrt_rn(sq3(__fsub_rn(px, qx), __fsub_rn(py, qy), __fsub_rn(pz, qz)));
                 } else {
                     float* gq = s_gt + (i >> 2) * 12 + (i & 3);
-                    gq[0] = SENTINEL;
-                    gq[4] = SENTINEL;
-                    gq[8] = SENTINEL;
+                    gq[0] = GT_SENTINEL;
+                    gq[4] = GT_SENTINEL;
+                    gq[8] = GT_SENTINEL;
                 }
             }
         }
@@ -496,7 +474,6 @@ static bool class_is_relaid(int cls) { return p6d_sched_state[16 + cls] == 't'; 
 //   0 = not checked yet, 1 = verified, 2 = rejected
 static std::atomic<int> g_relaid_state[64][3];
 static std::recursive_mutex g_config_mu;                // launch configuration + self-check (cold paths only)
-static size_t g_smem_raised[64][P6D_MAX_VARIANTS];   // per-device opt-in shared memory, only ever raised
 
 static bool relaid_disabled_by_env() {
     static const bool off = [] {
@@ -554,11 +531,42 @@ __global__ void quat_to_mat_kernel(const float* __restrict__ q, int64_t B, float
     for (int k = 0; k < 9; ++k) R[9 * b + k] = r[k];
 }
 
-static int max_optin_smem(int device, int* out) {
-    int v = 0;
-    P6D_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
-    *out = v;
+int max_optin_smem(int device, int* limit) {
+    static std::atomic<int> cached[64];   // 0 = not queried yet
+    std::atomic<int>& c = cached[device & 63];
+    int v = c.load(std::memory_order_relaxed);
+    if (v == 0) {
+        P6D_CUDA(cudaDeviceGetAttribute(&v, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
+        c.store(v, std::memory_order_relaxed);
+    }
+    *limit = v;
     return P6D_OK;
+}
+
+int raise_dyn_smem(const void* fn, int device, size_t bytes) {
+    // the attribute is a per-device maximum shared by every table and thread: lowering it for a smaller table would
+    // break a concurrent launch for a larger one
+    struct Raised { const void* fn; int device; size_t bytes; };
+    static std::mutex mu;
+    static std::vector<Raised> raised;
+    std::lock_guard<std::mutex> lock(mu);
+    auto it = std::find_if(raised.begin(), raised.end(), [&](const Raised& r) { return r.fn == fn && r.device == device; });
+    if (it == raised.end()) it = raised.insert(it, Raised{fn, device, 0});
+    if (bytes > it->bytes) {
+        P6D_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes)));
+        it->bytes = bytes;
+    }
+    return P6D_OK;
+}
+
+int claim_counter(const p6d_mesh_table* t, cudaStream_t st, int** counter) {
+    *counter = t->d_counters + (__atomic_fetch_add(&t->counter_idx, 1u, __ATOMIC_RELAXED) % P6D_NUM_COUNTERS);
+    P6D_CUDA(cudaMemsetAsync(*counter, 0, sizeof(int), st));
+    return P6D_OK;
+}
+
+static bool resident_fits(const p6d_mesh_table* t, int limit) {
+    return adds_smem_bytes(t->max_count) + 256 <= static_cast<size_t>(limit);
 }
 
 static int adds_max_points_for(int smem_limit) {
@@ -579,18 +587,14 @@ static int configure_variant(const p6d_mesh_table* t, int vi, size_t smem, int* 
     int limit = 0;
     int rc = max_optin_smem(t->device, &limit);
     if (rc) return rc;
-    if (smem + 256 > static_cast<size_t>(limit)) {
+    if (!resident_fits(t, limit)) {
         set_error("largest mesh has %d points; the ADD-S kernel holds the mesh, the gt cloud and two "
                   "distance rows in shared memory and accepts at most %d points on this device",
                   t->max_count, adds_max_points_for(limit));
         return P6D_ETOOBIG;
     }
     const AddsVariant& var = g_adds_variants[vi];
-    size_t& cur = g_smem_raised[t->device & 63][vi];
-    if (smem > cur) {
-        P6D_CUDA(cudaFuncSetAttribute(var.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-        cur = smem;
-    }
+    if ((rc = raise_dyn_smem(var.fn, t->device, smem))) return rc;
     int occ = 0;
     P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, var.fn, var.threads, smem));
     v = occ < 1 ? 1 : occ;
@@ -599,10 +603,6 @@ static int configure_variant(const p6d_mesh_table* t, int vi, size_t smem, int* 
     return P6D_OK;
 }
 
-// p6d_adds_streamed.cu: the opt-in kernel for meshes beyond shared memory (p6d_mesh_table_set_large_meshes)
-bool large_meshes_enabled(const p6d_mesh_table* t);
-int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st);
-
 void fill_eval_args(const p6d_mesh_table* t, EvalArgs& a) {
     a.soa = t->d_soa;
     a.pair = t->d_pair;
@@ -610,46 +610,8 @@ void fill_eval_args(const p6d_mesh_table* t, EvalArgs& a) {
     a.n_slots = t->n_slots;
 }
 
-int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st, int* launches,
-                int* grid_out, int force_variant) {
-    if (args.B == 0) return P6D_OK;
-    // poses are claimed through a 32-bit counter that runs up to B + grid
-    if (args.B > static_cast<int64_t>(INT32_MAX) - (1 << 20)) {
-        set_error("p6d_add_eval: B = %lld exceeds the per-launch limit of %d poses; split the batch",
-                  static_cast<long long>(args.B), INT32_MAX - (1 << 20));
-        return P6D_EINVAL;
-    }
-    if (!want_adds) {
-        const int rc = launch_add_only(t, args, st);
-        if (rc == P6D_OK && launches) ++*launches;
-        return rc;
-    }
-    if (force_variant < 0 && !args.sample) {
-        // opt-in (p6d_mesh_table_set_pruning): the exact-pruned kernel where the table qualifies
-        bool used = false;
-        const int rc = launch_eval_pruned(t, args, st, false, &used);
-        if (rc != P6D_OK) return rc;
-        if (used) {
-            if (launches) ++*launches;
-            return P6D_OK;
-        }
-        // opt-in (p6d_mesh_table_set_large_meshes): the streamed kernel, only where the resident one cannot run
-        if (large_meshes_enabled(t)) {
-            int limit = 0;
-            const int rc2 = max_optin_smem(t->device, &limit);
-            if (rc2) return rc2;
-            if (adds_smem_bytes(t->max_count) + 256 > static_cast<size_t>(limit)) {
-                const int rc3 = launch_eval_streamed(t, args, true, st);
-                if (rc3 == P6D_OK && launches) ++*launches;
-                return rc3;
-            }
-        }
-    }
-    int vi = force_variant;
-    if (vi < 0) {
-        const int rc = pick_variant(t, args.sample != nullptr, st, &vi);
-        if (rc) return rc;
-    }
+// The resident ADD-S kernel (b), variant vi
+static int launch_resident(const p6d_mesh_table* t, const EvalArgs& args, int vi, cudaStream_t st, int* grid_out) {
     const size_t smem = adds_smem_bytes(t->max_count);
     const AddsVariant& var = g_adds_variants[vi];
     int per_sm = 0;
@@ -665,15 +627,58 @@ int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, c
         a2.scan_reps = reps;
     }
 #endif
-    a2.work_counter = t->d_counters + (__atomic_fetch_add(&t->counter_idx, 1u, __ATOMIC_RELAXED) % P6D_NUM_COUNTERS);
-    P6D_CUDA(cudaMemsetAsync(a2.work_counter, 0, sizeof(int), st));
+    if ((rc = claim_counter(t, st, &a2.work_counter))) return rc;
     int nmax = t->max_count;
     void* kargs[] = {&a2, &nmax};
     P6D_CUDA(cudaLaunchKernel(var.fn, dim3(static_cast<unsigned>(grid)), dim3(var.threads), kargs, smem, st));
     P6D_CUDA(cudaGetLastError());
-    if (launches) ++*launches;
     if (grid_out) *grid_out = static_cast<int>(grid);
     return P6D_OK;
+}
+
+// largest mesh of a table below this: the pruned kernel has next to nothing to skip (1.05x at 37 points)
+constexpr int PR_MIN_POINTS = 128;
+
+// Every evaluation call (p6d_add_eval, p6d_add_eval_host, p6d_add_forward, p6d_sweep_run) picks its kernel here,
+// and only here:
+//   * a forced variant (the self-check) or the loss form: the resident ADD-S kernel (b), pick_variant's variant;
+//   * without ADD-S: the ADD-only kernel (a); beyond its shared memory, the streamed kernel if the table's large-mesh
+//     switch is on;
+//   * pruning switch on, a block structure, a largest mesh of >= PR_MIN_POINTS that fits: the pruned kernel;
+//   * large-mesh switch on and a mesh beyond the resident kernel's shared memory: the streamed kernel;
+//   * otherwise the resident ADD-S kernel.
+// Wherever two of these kernels can run a call, they give the same bytes.
+int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st, int* launches,
+                int* grid_out, int force_variant) {
+    if (args.B == 0) return P6D_OK;
+    // poses are claimed through a 32-bit counter that runs up to B + grid
+    if (args.B > static_cast<int64_t>(INT32_MAX) - (1 << 20)) {
+        set_error("p6d_add_eval: B = %lld exceeds the per-launch limit of %d poses; split the batch",
+                  static_cast<long long>(args.B), INT32_MAX - (1 << 20));
+        return P6D_EINVAL;
+    }
+    int rc = P6D_OK, vi = force_variant;
+    if (vi >= 0 || args.sample) {
+        if (vi < 0) rc = pick_variant(t, true, st, &vi);
+        if (rc == P6D_OK) rc = launch_resident(t, args, vi, st, grid_out);
+    } else {
+        const bool large = t->large_meshes.load(std::memory_order_relaxed);
+        const bool prune = want_adds && t->pruned && t->pruning.load(std::memory_order_relaxed) &&
+                           t->max_count >= PR_MIN_POINTS;
+        int limit = 0;
+        if ((large || prune) && (rc = max_optin_smem(t->device, &limit))) return rc;
+        if (!want_adds)
+            rc = large && !add_only_fits(t, limit) ? launch_eval_streamed(t, args, false, st)
+                                                   : launch_add_only(t, args, st);
+        else if (prune && pruned_fits(t, limit))
+            rc = launch_eval_pruned(t, args, st);
+        else if (large && !resident_fits(t, limit))
+            rc = launch_eval_streamed(t, args, true, st);
+        else if ((rc = pick_variant(t, false, st, &vi)) == P6D_OK)
+            rc = launch_resident(t, args, vi, st, grid_out);
+    }
+    if (rc == P6D_OK && launches) ++*launches;
+    return rc;
 }
 
 // The same n_poses seeded poses through the re-laid kernel and the ptxas kernel of class `cls`;
@@ -813,12 +818,6 @@ int p6d_adds_max_points(int device, int* max_points) {
     return P6D_OK;
 }
 
-// block structure of the opt-in pruned ADD-S kernel (p6d_adds_pruned.cu)
-void p6d_internal_build_pruned(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets);
-void p6d_internal_release_pruned(const p6d_mesh_table* t);
-// per-table switch of the streamed kernel (p6d_adds_streamed.cu)
-void p6d_internal_release_streamed(const p6d_mesh_table* t);
-
 int p6d_mesh_table_create(const float* xyz, const int32_t* offsets, const int32_t* counts,
                           const double* diameters, const uint8_t* symmetric, int n_slots, int device,
                           p6d_mesh_table** out) {
@@ -893,7 +892,7 @@ int p6d_mesh_table_create(const float* xyz, const int32_t* offsets, const int32_
         return fail(e, "cudaMemcpy(pair)");
     if ((e = cudaMemcpy(t->d_slots, t->h_slots, n_slots * sizeof(SlotInfo), cudaMemcpyHostToDevice)) != cudaSuccess)
         return fail(e, "cudaMemcpy(slots)");
-    p6d_internal_build_pruned(t, xyz, offsets);
+    t->pruned = build_pruned(t, xyz, offsets);
     *out = t;
     return P6D_OK;
 }
@@ -901,8 +900,7 @@ int p6d_mesh_table_create(const float* xyz, const int32_t* offsets, const int32_
 int p6d_mesh_table_destroy(p6d_mesh_table* t) {
     if (!t) return P6D_OK;
     DeviceGuard guard(t->device);
-    p6d_internal_release_pruned(t);
-    p6d_internal_release_streamed(t);
+    free_pruned(t->pruned);
     if (t->stream) cudaStreamDestroy(t->stream);
     if (t->d_stage) cudaFree(t->d_stage);
     if (t->h_pinned) cudaFreeHost(t->h_pinned);
@@ -915,30 +913,96 @@ int p6d_mesh_table_destroy(p6d_mesh_table* t) {
     return P6D_OK;
 }
 
+int p6d_mesh_table_set_pruning(p6d_mesh_table* table, int enable) {
+    if (!table) { set_error("p6d_mesh_table_set_pruning: table is NULL"); return P6D_EINVAL; }
+    if (!table->pruned) {
+        if (!enable) return P6D_OK;
+        set_error("p6d_mesh_table_set_pruning: this table has no block structure (a mesh with more than 65,534 points, "
+                  "or out of memory at creation)");
+        return P6D_ETOOBIG;
+    }
+    table->pruning.store(enable != 0, std::memory_order_relaxed);
+    return P6D_OK;
+}
+
+int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable) {
+    if (!table) { set_error("p6d_mesh_table_set_large_meshes: table is NULL"); return P6D_EINVAL; }
+    table->large_meshes.store(enable != 0, std::memory_order_relaxed);
+    return P6D_OK;
+}
+
+}  // extern "C"
+
 // float4 / float2 / int4 loads in the kernels need their natural alignment
 static bool misaligned(const void* p, size_t a) { return p && (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
+
+// Argument checks of the device-buffer evaluation entries (messages prefixed with `fn`), then *a.  need_adds: the
+// entry computes ADD-S in any case (p6d_add_eval_pruned).
+static int eval_entry_args(const char* fn, bool need_adds, const p6d_mesh_table* table, const float* pq,
+                           const float* pt, const float* gq, const float* gt, const int64_t* obj, const int32_t* order,
+                           int64_t B, float* add, float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                           const p6d_accumulators* acc, EvalArgs* a) {
+    if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || (need_adds && !adds) || !hit || !valid))) {
+        set_error("%s: bad arguments", fn);
+        return P6D_EINVAL;
+    }
+    if (misaligned(pq, 4) || misaligned(pt, 4) || misaligned(gq, 4) || misaligned(gt, 4) || misaligned(obj, 8) ||
+        misaligned(order, 4) || misaligned(add, 4) || misaligned(adds, 4)) {
+        set_error("%s: a pointer is not aligned to its element size", fn);
+        return P6D_EINVAL;
+    }
+    if (B > static_cast<int64_t>(INT32_MAX) - (1 << 20)) {
+        set_error("%s: B = %lld exceeds the per-launch limit of %d poses; split the batch", fn,
+                  static_cast<long long>(B), INT32_MAX - (1 << 20));
+        return P6D_EINVAL;
+    }
+    *a = EvalArgs{};
+    fill_eval_args(table, *a);
+    a->pq = pq; a->pt = pt; a->gq = gq; a->gt = gt; a->obj = obj; a->order = order; a->B = B;
+    a->add = add; a->adds = adds; a->hit = hit; a->valid = valid; a->borderline = borderline;
+    if (acc) { a->acc = *acc; a->has_acc = 1; }
+    return P6D_OK;
+}
+
+extern "C" {
 
 int p6d_add_eval(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                  const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
                  float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                  const p6d_accumulators* acc, void* stream) {
-    if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || !hit || !valid))) {
-        set_error("p6d_add_eval: bad arguments");
-        return P6D_EINVAL;
-    }
-    if (misaligned(pq, 4) || misaligned(pt, 4) || misaligned(gq, 4) || misaligned(gt, 4) || misaligned(obj, 8) ||
-        misaligned(order, 4) || misaligned(add, 4) || misaligned(adds, 4)) {
-        set_error("p6d_add_eval: a pointer is not aligned to its element size");
-        return P6D_EINVAL;
-    }
+    EvalArgs a;
+    const int rc = eval_entry_args("p6d_add_eval", false, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid,
+                                   borderline, acc, &a);
+    if (rc != P6D_OK || B == 0) return rc;
     DeviceGuard guard(table->device);
     if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    EvalArgs a{};
-    fill_eval_args(table, a);
-    a.pq = pq; a.pt = pt; a.gq = gq; a.gt = gt; a.obj = obj; a.order = order; a.B = B;
-    a.add = add; a.adds = adds; a.hit = hit; a.valid = valid; a.borderline = borderline;
-    if (acc) { a.acc = *acc; a.has_acc = 1; }
     return launch_eval(table, a, adds != nullptr, static_cast<cudaStream_t>(stream), nullptr);
+}
+
+int p6d_add_eval_pruned(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                        const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
+                        float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                        const p6d_accumulators* acc, void* stream) {
+    EvalArgs a;
+    const int rc = eval_entry_args("p6d_add_eval_pruned", true, table, pq, pt, gq, gt, obj, order, B, add, adds, hit,
+                                   valid, borderline, acc, &a);
+    if (rc != P6D_OK || B == 0) return rc;
+    DeviceGuard guard(table->device);
+    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
+    return launch_eval_pruned(table, a, static_cast<cudaStream_t>(stream));
+}
+
+int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                          const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
+                          float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                          const p6d_accumulators* acc, void* stream) {
+    EvalArgs a;
+    const int rc = eval_entry_args("p6d_add_eval_streamed", false, table, pq, pt, gq, gt, obj, order, B, add, adds,
+                                   hit, valid, borderline, acc, &a);
+    if (rc != P6D_OK || B == 0) return rc;
+    DeviceGuard guard(table->device);
+    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
+    return launch_eval_streamed(table, a, adds != nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int64_t p6d_add_forward_workspace_bytes(const p6d_mesh_table* table, int64_t B) {

@@ -10,7 +10,6 @@
 //   loss = (1/count) * sum_b mean_i d_bi ,  d = |p_i - g_i| (ADD) or min_j |p_i - g_j| (ADD-S)
 //   dL/dp_i = scale * (p_i - g*) / d   (0 where d == 0, PyTorch's norm sub-gradient)
 // Training-size problem (B = 32, N = 500): latency matters, throughput does not.
-#include <mutex>
 
 #include "p6d_common.cuh"
 
@@ -171,22 +170,13 @@ extern "C" int p6d_add_backward(const p6d_mesh_table* table, const float* pq, co
     const int nmax = table->max_count > 0 ? table->max_count : 1;
     const size_t smem = sizeof(float) * 3 * (size_t)nmax;
     int limit = 0;
-    P6D_CUDA(cudaDeviceGetAttribute(&limit, cudaDevAttrMaxSharedMemoryPerBlockOptin, table->device));
+    int rc = max_optin_smem(table->device, &limit);
+    if (rc) return rc;
     if (smem + 1024 > (size_t)limit) {
         set_error("p6d_add_backward: mesh of %d points does not fit shared memory", nmax);
         return P6D_ETOOBIG;
     }
-    {
-        // the attribute is a per-device maximum shared by every table and thread: only ever raise it
-        static std::mutex mu;
-        static size_t raised[64];
-        std::lock_guard<std::mutex> lock(mu);
-        size_t& cur = raised[table->device & 63];
-        if (smem > cur) {
-            P6D_CUDA(cudaFuncSetAttribute(add_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            cur = smem;
-        }
-    }
+    if ((rc = raise_dyn_smem((const void*)add_backward_kernel, table->device, smem))) return rc;
     BwdArgs a{table->d_soa, table->d_slots, table->n_slots, pq, pt, gq, gt, obj, B, grad_out, count, inv_count, grad_q, grad_t};
     int64_t grid = B < (int64_t)table->sm_count * 4 ? B : (int64_t)table->sm_count * 4;
     add_backward_kernel<<<(unsigned)grid, BWD_T, smem, static_cast<cudaStream_t>(stream)>>>(a, nmax);

@@ -27,10 +27,7 @@
 // The squared distance of a pair is computed by the same packed instructions in the same order as kernel (b)
 // (3 FADD2, FMUL2, 2 FFMA2, FMNMX3.NAN), so every surviving value has the same bits.
 #include <algorithm>
-#include <atomic>
-#include <map>
 #include <memory>
-#include <mutex>
 #include <vector>
 
 #include "p6d_common.cuh"
@@ -39,8 +36,6 @@ namespace p6d {
 
 constexpr int PR_BLOCK = 32;              // points per block = lanes per warp
 constexpr int PR_SUB = 8;                 // points per gt sub-block (two quads)
-constexpr float PR_SENTINEL = 1.0e18f;    // padded gt coordinate: never the minimum (as in kernel (b))
-constexpr int PR_MIN_POINTS = 128;        // largest mesh of a table below this: nothing to gain (1.05x at 37 points)
 
 // per-object description of the block-sorted copy of the mesh (device + host)
 struct PrunedSlot {
@@ -64,11 +59,7 @@ struct PrunedTable {
     std::vector<PrunedSlot> h_slots;
     int max_nb = 0;
     int max_count = 0;
-    std::atomic<bool> enabled{false};   // p6d_mesh_table_set_pruning: launch_eval takes this kernel where the table qualifies
 };
-
-static std::mutex g_pr_mu;
-static std::map<const p6d_mesh_table*, PrunedTable*> g_pr_tables;
 
 // k-d median splits: idx[lo, hi) -> blocks of 32 consecutive entries made of sub-blocks of 8, each spatially compact
 static void kd_split(const float* xyz, std::vector<int>& idx, int lo, int hi) {
@@ -95,7 +86,7 @@ static void kd_split(const float* xyz, std::vector<int>& idx, int lo, int hi) {
     kd_split(xyz, idx, mid, hi);
 }
 
-static PrunedTable* build_pruned(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets) {
+static PrunedTable* build_blocks(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets) {
     std::unique_ptr<PrunedTable> pt(new PrunedTable());     // freed if anything below throws
     pt->h_slots.resize(t->n_slots);
     size_t total = 0;
@@ -161,16 +152,19 @@ static PrunedTable* build_pruned(const p6d_mesh_table* t, const float* xyz, cons
     return pt.release();
 }
 
-// called by p6d_mesh_table_destroy
-void pruned_table_release(const p6d_mesh_table* t) {
-    PrunedTable* pt = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(g_pr_mu);
-        auto it = g_pr_tables.find(t);
-        if (it == g_pr_tables.end()) return;
-        pt = it->second;
-        g_pr_tables.erase(it);
+// Called by p6d_mesh_table_create once the table is complete.  Null (no block structure) for a mesh of more than
+// 65,534 points, or out of memory: not fatal for the table, the pruned kernel is just not available.
+PrunedTable* build_pruned(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets) {
+    if (t->max_count > 65534) return nullptr;    // permutation is stored as uint16
+    try {
+        return build_blocks(t, xyz, offsets);
+    } catch (...) {                              // out of host memory
+        return nullptr;
     }
+}
+
+void free_pruned(PrunedTable* pt) {
+    if (!pt) return;
     cudaFree(pt->d_sorted);
     cudaFree(pt->d_slots);
     delete pt;
@@ -194,42 +188,20 @@ __device__ __forceinline__ float eval_block(const float4* __restrict__ q, float 
 #pragma unroll
     for (int k = 0; k < PR_BLOCK / 4; ++k) {
         const float4 X = q[3 * k], Y = q[3 * k + 1], Z = q[3 * k + 2];
-        const float2 pxx = make_float2(px, px), pyy = make_float2(py, py), pzz = make_float2(pz, pz);
-        {
-            const float2 dx = sub2(pxx, make_float2(X.x, X.y)), dy = sub2(pyy, make_float2(Y.x, Y.y)),
-                         dz = sub2(pzz, make_float2(Z.x, Z.y));
-            const float2 s = fma2(dz, dz, fma2(dy, dy, mul2(dx, dx)));
-            m = min3_nan(m, s.x, s.y);
-        }
-        {
-            const float2 dx = sub2(pxx, make_float2(X.z, X.w)), dy = sub2(pyy, make_float2(Y.z, Y.w)),
-                         dz = sub2(pzz, make_float2(Z.z, Z.w));
-            const float2 s = fma2(dz, dz, fma2(dy, dy, mul2(dx, dx)));
-            m2 = min3_nan(m2, s.x, s.y);
-        }
+        pair_tile(px, py, pz, make_float2(X.x, X.y), make_float2(Y.x, Y.y), make_float2(Z.x, Z.y), m);
+        pair_tile(px, py, pz, make_float2(X.z, X.w), make_float2(Y.z, Y.w), make_float2(Z.z, Z.w), m2);
     }
     return min_nan(m, m2);
 }
 
 // one gt sub-block (2 quads) against the lane's pred point
 __device__ __forceinline__ float eval_sub(const float4* __restrict__ q, float px, float py, float pz, float m) {
-    const float2 pxx = make_float2(px, px), pyy = make_float2(py, py), pzz = make_float2(pz, pz);
     float m2 = __int_as_float(0x7f800000);
 #pragma unroll
     for (int k = 0; k < PR_SUB / 4; ++k) {
         const float4 X = q[3 * k], Y = q[3 * k + 1], Z = q[3 * k + 2];
-        {
-            const float2 dx = sub2(pxx, make_float2(X.x, X.y)), dy = sub2(pyy, make_float2(Y.x, Y.y)),
-                         dz = sub2(pzz, make_float2(Z.x, Z.y));
-            const float2 s = fma2(dz, dz, fma2(dy, dy, mul2(dx, dx)));
-            m = min3_nan(m, s.x, s.y);
-        }
-        {
-            const float2 dx = sub2(pxx, make_float2(X.z, X.w)), dy = sub2(pyy, make_float2(Y.z, Y.w)),
-                         dz = sub2(pzz, make_float2(Z.z, Z.w));
-            const float2 s = fma2(dz, dz, fma2(dy, dy, mul2(dx, dx)));
-            m2 = min3_nan(m2, s.x, s.y);
-        }
+        pair_tile(px, py, pz, make_float2(X.x, X.y), make_float2(Y.x, Y.y), make_float2(Z.x, Z.y), m);
+        pair_tile(px, py, pz, make_float2(X.z, X.w), make_float2(Y.z, Y.w), make_float2(Z.z, Z.w), m2);
     }
     return min_nan(m, m2);
 }
@@ -351,9 +323,9 @@ __global__ void __launch_bounds__(T, MINB) adds_pruned_kernel(EvalArgs a, Pruned
                 s_pred[np + p] = py;
                 s_pred[2 * np + p] = pz;
                 float* gq = s_gt + (p >> 2) * 12 + (p & 3);
-                gq[0] = valid ? qx : PR_SENTINEL;
-                gq[4] = valid ? qy : PR_SENTINEL;
-                gq[8] = valid ? qz : PR_SENTINEL;
+                gq[0] = valid ? qx : GT_SENTINEL;
+                gq[4] = valid ? qy : GT_SENTINEL;
+                gq[8] = valid ? qz : GT_SENTINEL;
                 if (valid) s_dadd[orig] = __fsqrt_rn(sq3(__fsub_rn(px, qx), __fsub_rn(py, qy), __fsub_rn(pz, qz)));
                 // spheres: centre = the transformed centroid (any point would do), radius from the actual points
                 const float cx = cen[blk], cy = cen[nbp + blk], cz = cen[2 * nbp + blk];
@@ -451,45 +423,40 @@ __global__ void __launch_bounds__(T, MINB) adds_pruned_kernel(EvalArgs a, Pruned
     }
 }
 
-static size_t g_pr_smem_raised[64];
+// dynamic shared memory of the table's largest mesh
+static size_t pruned_smem_bytes(const p6d_mesh_table* t) {
+    const int nb = t->pruned->max_nb > 0 ? t->pruned->max_nb : 1;
+    return sizeof(float) * pr_smem_floats(nb, t->max_count);
+}
 
-// The pruned kernel for one evaluation launch.  force = the explicit entry point (any mesh size that fits);
-// otherwise only when the table's switch is on and the table qualifies: below PR_MIN_POINTS there is next to
-// nothing to skip, and a mesh that does not fit this kernel's shared memory takes the all-pairs kernel as well.
-// *used tells the caller whether a launch happened.
-int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaStream_t st, bool force, bool* used) {
-    *used = false;
-    PrunedTable* ptab = nullptr;
-    {
-        std::lock_guard<std::mutex> lock(g_pr_mu);
-        auto it = g_pr_tables.find(table);
-        if (it != g_pr_tables.end()) ptab = it->second;
+bool pruned_fits(const p6d_mesh_table* t, int limit) {   // t has a block structure
+    return pruned_smem_bytes(t) + 1024 <= static_cast<size_t>(limit);
+}
+
+// The pruned kernel for one evaluation launch, for any mesh size that fits (launch_eval decides when it pays).
+int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaStream_t st) {
+    const PrunedTable* ptab = table->pruned;
+    if (!ptab) {
+        set_error("p6d_add_eval_pruned: this table has no block structure (a mesh with more than 65,534 points, or out of "
+                  "memory at creation)");
+        return P6D_ETOOBIG;
     }
-    if (!ptab || (!force && (!ptab->enabled.load(std::memory_order_relaxed) || table->max_count < PR_MIN_POINTS))) return P6D_OK;
+    int limit = 0;
+    int rc = max_optin_smem(table->device, &limit);
+    if (rc) return rc;
+    if (!pruned_fits(table, limit)) {
+        set_error("largest mesh has %d points; the pruned ADD-S kernel keeps both clouds and the sorted mesh in "
+                  "shared memory and accepts at most %d points on this device (p6d_add_eval takes larger meshes)",
+                  table->max_count, (limit - 1024) / 4 / 12 / 32 * 32);
+        return P6D_ETOOBIG;
+    }
     const int nb = ptab->max_nb > 0 ? ptab->max_nb : 1;
-    const size_t smem = sizeof(float) * pr_smem_floats(nb, table->max_count);
-    {
-        std::lock_guard<std::mutex> lock(g_pr_mu);
-        size_t& cur = g_pr_smem_raised[table->device & 63];
-        if (smem > cur) {
-            int limit = 0;
-            P6D_CUDA(cudaDeviceGetAttribute(&limit, cudaDevAttrMaxSharedMemoryPerBlockOptin, table->device));
-            if (smem + 1024 > static_cast<size_t>(limit)) {
-                if (!force) return P6D_OK;
-                set_error("largest mesh has %d points; the pruned ADD-S kernel keeps both clouds and the sorted mesh in "
-                          "shared memory and accepts at most %d points on this device (p6d_add_eval takes larger meshes)",
-                          table->max_count, (limit - 1024) / 4 / 12 / 32 * 32);
-                return P6D_ETOOBIG;
-            }
-            for (const void* fn : {(const void*)adds_pruned_kernel<256, 2>, (const void*)adds_pruned_kernel<256, 3>,
-                                   (const void*)adds_pruned_kernel<256, 4>, (const void*)adds_pruned_kernel<128, 8>})
-                P6D_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-            cur = smem;
-        }
-    }
+    const size_t smem = pruned_smem_bytes(table);
+    for (const void* fn : {(const void*)adds_pruned_kernel<256, 2>, (const void*)adds_pruned_kernel<256, 3>,
+                           (const void*)adds_pruned_kernel<256, 4>, (const void*)adds_pruned_kernel<128, 8>})
+        if ((rc = raise_dyn_smem(fn, table->device, smem))) return rc;
     EvalArgs a = args;
-    a.work_counter = table->d_counters + (__atomic_fetch_add(&table->counter_idx, 1u, __ATOMIC_RELAXED) % P6D_NUM_COUNTERS);
-    P6D_CUDA(cudaMemsetAsync(a.work_counter, 0, sizeof(int), st));
+    if ((rc = claim_counter(table, st, &a.work_counter))) return rc;
     // the instantiation whose register budget matches what shared memory lets be resident (see the kernel's comment)
     struct Shape { const void* fn; int threads, minb; };
     const Shape shapes[] = {{(const void*)adds_pruned_kernel<128, 8>, 128, 8}, {(const void*)adds_pruned_kernel<256, 4>, 256, 4},
@@ -514,81 +481,7 @@ int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaSt
     void* kargs[] = {&a, &pa, &nb_arg, &nmax_arg};
     P6D_CUDA(cudaLaunchKernel(pick->fn, dim3(static_cast<unsigned>(grid)), dim3(pick->threads), kargs, smem, st));
     P6D_CUDA(cudaGetLastError());
-    *used = true;
     return P6D_OK;
 }
 
 }  // namespace p6d
-
-using namespace p6d;
-
-extern "C" {
-
-// Called by p6d_mesh_table_create once the table is complete.  Failure is not fatal for the table: the pruned
-// entry point then reports that the table has no blocks.
-void p6d_internal_build_pruned(const p6d_mesh_table* t, const float* xyz, const int32_t* offsets) {
-    if (t->max_count > 65534) return;            // permutation is stored as uint16
-    PrunedTable* pt = nullptr;
-    try {
-        pt = build_pruned(t, xyz, offsets);
-    } catch (...) {                              // out of host memory: the table simply has no blocks
-        return;
-    }
-    if (!pt) return;
-    std::lock_guard<std::mutex> lock(g_pr_mu);
-    g_pr_tables[t] = pt;
-}
-
-void p6d_internal_release_pruned(const p6d_mesh_table* t) { pruned_table_release(t); }
-
-int p6d_mesh_table_set_pruning(p6d_mesh_table* table, int enable) {
-    if (!table) { set_error("p6d_mesh_table_set_pruning: table is NULL"); return P6D_EINVAL; }
-    std::lock_guard<std::mutex> lock(g_pr_mu);
-    auto it = g_pr_tables.find(table);
-    if (it == g_pr_tables.end()) {
-        if (!enable) return P6D_OK;
-        set_error("p6d_mesh_table_set_pruning: this table has no block structure (a mesh with more than 65,534 points, "
-                  "or out of memory at creation)");
-        return P6D_ETOOBIG;
-    }
-    it->second->enabled.store(enable != 0, std::memory_order_relaxed);
-    return P6D_OK;
-}
-
-int p6d_add_eval_pruned(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
-                        const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
-                        float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
-                        const p6d_accumulators* acc, void* stream) {
-    if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || !adds || !hit || !valid))) {
-        set_error("p6d_add_eval_pruned: bad arguments");
-        return P6D_EINVAL;
-    }
-    auto mis = [](const void* p, size_t al) { return p && (reinterpret_cast<uintptr_t>(p) & (al - 1)) != 0; };
-    if (mis(pq, 4) || mis(pt, 4) || mis(gq, 4) || mis(gt, 4) || mis(obj, 8) || mis(order, 4) || mis(add, 4) || mis(adds, 4)) {
-        set_error("p6d_add_eval_pruned: a pointer is not aligned to its element size");
-        return P6D_EINVAL;
-    }
-    if (B == 0) return P6D_OK;
-    if (B > static_cast<int64_t>(INT32_MAX) - (1 << 20)) {
-        set_error("p6d_add_eval_pruned: B = %lld exceeds the per-launch limit of %d poses; split the batch",
-                  static_cast<long long>(B), INT32_MAX - (1 << 20));
-        return P6D_EINVAL;
-    }
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    EvalArgs a{};
-    fill_eval_args(table, a);
-    a.pq = pq; a.pt = pt; a.gq = gq; a.gt = gt; a.obj = obj; a.order = order; a.B = B;
-    a.add = add; a.adds = adds; a.hit = hit; a.valid = valid; a.borderline = borderline;
-    if (acc) { a.acc = *acc; a.has_acc = 1; }
-    bool used = false;
-    const int rc = launch_eval_pruned(table, a, static_cast<cudaStream_t>(stream), true, &used);
-    if (rc == P6D_OK && !used) {
-        set_error("p6d_add_eval_pruned: this table has no block structure (a mesh with more than 65,534 points, or out of "
-                  "memory at creation)");
-        return P6D_ETOOBIG;
-    }
-    return rc;
-}
-
-}  // extern "C"

@@ -11,7 +11,7 @@
 //                with the slot's torch.mm rounding), plus the gt point of the same index for the ADD distance;
 //   gt side    = tiles of G = 1,024 mesh points arrive by TMA bulk copies (x, y, z segments of the table's SoA
 //                block) in a two-stage mbarrier ring, are transformed by the gt pose into the quad layout of
-//                kernel (b) (padded with SENTINEL) and scanned with its packed step (3 FADD2 + FMUL2 + 2 FFMA2 +
+//                kernel (b) (padded with GT_SENTINEL) and scanned with its packed step (3 FADD2 + FMUL2 + 2 FFMA2 +
 //                FMNMX3.NAN per two pairs).  The gt cloud is re-transformed per item: 18 FLOP per gt point against
 //                8 * P per gt point of scan, so nothing per pose goes through global memory;
 //   finish     = sqrt of each row minimum (sqrt is monotone and correctly rounded, and min is exact and
@@ -23,8 +23,6 @@
 // the batch is launched in chunks that keep it within 64 MB, so two streams never share a buffer.
 #include <algorithm>
 #include <atomic>
-#include <mutex>
-#include <set>
 
 #include "p6d_common.cuh"
 
@@ -35,7 +33,6 @@ constexpr int ST_G = 1024;                 // gt points per tile (multiple of 8)
 constexpr int ST_STAGES = 2;               // TMA ring depth
 constexpr int ST_MAX_POINTS = 32768;       // see the refusal message in launch_eval_streamed
 constexpr size_t ST_WS_BYTES = size_t(64) << 20;
-constexpr float ST_SENTINEL = 1.0e18f;     // padded gt coordinate: never the minimum (as in kernel (b))
 
 struct StreamArgs {
     int64_t first;      // first pose of the chunk in processing order
@@ -46,17 +43,6 @@ struct StreamArgs {
     int* tickets;       // [nposes] finished items per pose (zeroed before the launch)
     float* rows;        // [nposes][2][stride]: ADD row, ADD-S row
 };
-
-__device__ __forceinline__ void st_pair_tile(float px, float py, float pz, float2 gx, float2 gy, float2 gz, float& m) {
-    // two (pred, gt) pairs: the arithmetic of kernel (b), operation for operation
-    const float2 dx = sub2(make_float2(px, px), gx);
-    const float2 dy = sub2(make_float2(py, py), gy);
-    const float2 dz = sub2(make_float2(pz, pz), gz);
-    float2 s = mul2(dx, dx);
-    s = fma2(dy, dy, s);
-    s = fma2(dz, dz, s);
-    m = min3_nan(m, s.x, s.y);
-}
 
 template <int K, int MINB, bool ADDS>
 __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, StreamArgs sa) {
@@ -176,9 +162,9 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
                         gq[4] = qy;
                         gq[8] = qz;
                     } else {
-                        gq[0] = ST_SENTINEL;
-                        gq[4] = ST_SENTINEL;
-                        gq[8] = ST_SENTINEL;
+                        gq[0] = GT_SENTINEL;
+                        gq[4] = GT_SENTINEL;
+                        gq[8] = GT_SENTINEL;
                     }
                 }
                 __syncthreads();  // (T2) s_quad is complete and s_raw[st] is consumed
@@ -193,14 +179,14 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
                     const float4 X0 = p[0], Y0 = p[1], Z0 = p[2], X1 = p[3], Y1 = p[4], Z1 = p[5];
 #pragma unroll
                     for (int k = 0; k < K; ++k) {
-                        st_pair_tile(px[k], py[k], pz[k], make_float2(X0.x, X0.y), make_float2(Y0.x, Y0.y),
-                                     make_float2(Z0.x, Z0.y), m[k]);
-                        st_pair_tile(px[k], py[k], pz[k], make_float2(X0.z, X0.w), make_float2(Y0.z, Y0.w),
-                                     make_float2(Z0.z, Z0.w), m[k]);
-                        st_pair_tile(px[k], py[k], pz[k], make_float2(X1.x, X1.y), make_float2(Y1.x, Y1.y),
-                                     make_float2(Z1.x, Z1.y), m[k]);
-                        st_pair_tile(px[k], py[k], pz[k], make_float2(X1.z, X1.w), make_float2(Y1.z, Y1.w),
-                                     make_float2(Z1.z, Z1.w), m[k]);
+                        pair_tile(px[k], py[k], pz[k], make_float2(X0.x, X0.y), make_float2(Y0.x, Y0.y),
+                                  make_float2(Z0.x, Z0.y), m[k]);
+                        pair_tile(px[k], py[k], pz[k], make_float2(X0.z, X0.w), make_float2(Y0.z, Y0.w),
+                                  make_float2(Z0.z, Z0.w), m[k]);
+                        pair_tile(px[k], py[k], pz[k], make_float2(X1.x, X1.y), make_float2(Y1.x, Y1.y),
+                                  make_float2(Z1.x, Z1.y), m[k]);
+                        pair_tile(px[k], py[k], pz[k], make_float2(X1.z, X1.w), make_float2(Y1.z, Y1.w),
+                                  make_float2(Z1.z, Z1.w), m[k]);
                     }
                 }
             }
@@ -254,14 +240,6 @@ static const StShape kStShapes[2][3] = {
      {(const void*)adds_streamed_kernel<2, 4, true>, 2}},
 };
 static std::atomic<int> g_st_per_sm[64][2][3];   // CTAs per SM (0 = not computed yet)
-
-static std::mutex g_st_mu;
-static std::set<const p6d_mesh_table*> g_st_enabled;   // tables with p6d_mesh_table_set_large_meshes on
-
-bool large_meshes_enabled(const p6d_mesh_table* t) {
-    std::lock_guard<std::mutex> lock(g_st_mu);
-    return g_st_enabled.count(t) != 0;
-}
 
 int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st) {
     if (t->max_count > ST_MAX_POINTS) {
@@ -332,51 +310,3 @@ int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool wan
 }
 
 }  // namespace p6d
-
-using namespace p6d;
-
-extern "C" {
-
-void p6d_internal_release_streamed(const p6d_mesh_table* t) {
-    std::lock_guard<std::mutex> lock(g_st_mu);
-    g_st_enabled.erase(t);
-}
-
-int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable) {
-    if (!table) { set_error("p6d_mesh_table_set_large_meshes: table is NULL"); return P6D_EINVAL; }
-    std::lock_guard<std::mutex> lock(g_st_mu);
-    if (enable) g_st_enabled.insert(table);
-    else g_st_enabled.erase(table);
-    return P6D_OK;
-}
-
-int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
-                          const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
-                          float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
-                          const p6d_accumulators* acc, void* stream) {
-    if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || !hit || !valid))) {
-        set_error("p6d_add_eval_streamed: bad arguments");
-        return P6D_EINVAL;
-    }
-    auto mis = [](const void* p, size_t al) { return p && (reinterpret_cast<uintptr_t>(p) & (al - 1)) != 0; };
-    if (mis(pq, 4) || mis(pt, 4) || mis(gq, 4) || mis(gt, 4) || mis(obj, 8) || mis(order, 4) || mis(add, 4) || mis(adds, 4)) {
-        set_error("p6d_add_eval_streamed: a pointer is not aligned to its element size");
-        return P6D_EINVAL;
-    }
-    if (B == 0) return P6D_OK;
-    if (B > static_cast<int64_t>(INT32_MAX) - (1 << 20)) {
-        set_error("p6d_add_eval_streamed: B = %lld exceeds the per-launch limit of %d poses; split the batch",
-                  static_cast<long long>(B), INT32_MAX - (1 << 20));
-        return P6D_EINVAL;
-    }
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    EvalArgs a{};
-    fill_eval_args(table, a);
-    a.pq = pq; a.pt = pt; a.gq = gq; a.gt = gt; a.obj = obj; a.order = order; a.B = B;
-    a.add = add; a.adds = adds; a.hit = hit; a.valid = valid; a.borderline = borderline;
-    if (acc) { a.acc = *acc; a.has_acc = 1; }
-    return launch_eval_streamed(table, a, adds != nullptr, static_cast<cudaStream_t>(stream));
-}
-
-}  // extern "C"
