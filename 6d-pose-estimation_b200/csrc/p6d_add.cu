@@ -224,11 +224,6 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
     // at the end.  One atomic per pose, issued one pose ahead so its latency is never exposed.
     // (Claiming several poses per atomic for small meshes was tried: it costs registers in
     // the scan loop and gains < 4 % at N = 500.)
-#ifdef P6D_DEV
-    unsigned long long t_start = 0;
-    int done = 0;
-    if (a.timeline && tid == 0) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_start));
-#endif
     if (tid == 0) s_next = atomicAdd(a.work_counter, 1);
     __syncthreads();
 
@@ -236,41 +231,19 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
         const int64_t it = s_next;
         if (it >= a.B) break;
         const int64_t b = a.order ? a.order[it] : it;
-        if (tid < 4) s_pose[tid] = __ldg(a.pq + 4 * b + tid);
-        else if (tid < 8) s_pose[tid] = __ldg(a.gq + 4 * b + tid - 4);
-        else if (tid < 11) s_pose[tid] = __ldg(a.pt + 3 * b + tid - 8);
-        else if (tid < 14) s_pose[tid] = __ldg(a.gt + 3 * b + tid - 11);
-        else if (tid == 32) s_oid = a.obj[b];
+        load_pose(a, b, tid, s_pose, &s_oid);
         __syncthreads();  // (A) also: previous pose's readers of s_gt / s_dadd* / s_mean / s_next are done
         if (tid == 64) s_next = atomicAdd(a.work_counter, 1);  // read after barriers (B) and (C)
-#ifdef P6D_DEV
-        ++done;
-#endif
         const long long oid = s_oid;
-        const bool known = oid >= 0 && oid < a.n_slots && a.slots[oid].count > 0;
-        if (!known) {  // CTA-uniform
-            if (tid == 0) {
-                a.add[b] = 0.0f;
-                a.adds[b] = 0.0f;
-                a.hit[b] = 0;
-                a.valid[b] = 0;
-                if (a.borderline) a.borderline[b] = 0;
-                if (LOSS) a.sample[b] = 0.0f;
-            }
+        if (!slot_known(oid, a.n_slots, a.slots)) {  // CTA-uniform
+            if (tid == 0) write_skipped<LOSS>(a, b, true);
             __syncthreads();
             continue;
         }
         const SlotInfo s = a.slots[oid];
         const int n = s.count, np = s.padded;
         if (oid != staged_oid) {
-            // stage the mesh: one elected thread arms the barrier and issues the bulk copy
-            if (tid == 0) {
-                fence_proxy_async();
-                const uint32_t bytes = 3u * static_cast<uint32_t>(np) * sizeof(float);
-                mbar_arrive_expect_tx(s_bar, bytes);
-                tma_bulk_g2s(s_mesh, a.soa + s.soa_offset, bytes, s_bar);
-            }
-            mbar_wait(s_bar, phase);
+            stage_mesh(s_mesh, a.soa + s.soa_offset, 3 * np, s_bar, phase, tid);
             phase ^= 1;
             staged_oid = oid;
         }
@@ -320,9 +293,6 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
         const int g = tid / S, sp = tid % S;
         const float4* gq4 = reinterpret_cast<const float4*>(s_gt);   // quad q at gq4[3q .. 3q+2]
         const int nquads = ng >> 2;
-#ifdef P6D_DEV
-        for (int rep = 0; rep < a.scan_reps; ++rep)
-#endif
         for (int base = 0; base < n; base += groups * K) {
             float px[K], py[K], pz[K], m[K];
             {
@@ -374,22 +344,8 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
 
         // phase D: ordered means (ATen summation order) on warps 0 and 1, decision, outputs
         if (tid < 64) {
-            const float* src = tid < 32 ? s_dadd : s_dadds;
-            const float mean = aten_mean_warp([&](int e) { return src[e]; }, n, lane);
-            if (lane == 0) s_mean[tid >> 5] = mean;
-            asm volatile("bar.sync 1, 64;" ::: "memory");
-            if (tid == 0) {
-                const float add = s_mean[0], adds = s_mean[1];
-                const float eff = s.symmetric ? adds : add;
-                const bool is_hit = static_cast<double>(eff) < s.threshold;
-                a.add[b] = add;
-                a.adds[b] = adds;
-                a.hit[b] = is_hit ? 1 : 0;
-                a.valid[b] = 1;
-                if (a.borderline) a.borderline[b] = near_threshold(eff, s.threshold) ? 1 : 0;
-                if (LOSS) a.sample[b] = eff;
-                accumulate(a, oid, is_hit, add, adds, true);
-            }
+            ordered_means(s_dadd, s_dadds, n, tid, lane, true, s_mean, [](const float* p) { return *p; });
+            if (tid == 0) write_pose<LOSS>(a, b, oid, s, s_mean[0], s_mean[1], true);
         }
         // barrier (A) of the next pose protects s_gt / s_dadd* / s_mean
     }
@@ -405,16 +361,6 @@ __global__ void __launch_bounds__(T, MINB) adds_cta_kernel(EvalArgs a, int nmax)
             loss_finalize<T>(a, tid);
         }
     }
-#ifdef P6D_DEV
-    if (a.timeline && tid == 0) {
-        unsigned long long t_end;
-        unsigned smid;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_end));
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        unsigned long long* o = a.timeline + 4ull * blockIdx.x;
-        o[0] = smid; o[1] = t_start; o[2] = t_end; o[3] = (unsigned long long)done;
-    }
-#endif
 }
 
 // Kernel variants.  Three mesh-size classes (N <= 512, <= 1024, larger), each with the shape ptxas
@@ -439,17 +385,7 @@ static const AddsVariant g_adds_variants[] = {
     {"T512_K4_B2_U2_loss", 512, (const void*)adds_cta_kernel<512, 4, 2, 2, 1>},
     {"T256_K4_B4_U2_loss", 256, (const void*)adds_cta_kernel<256, 4, 4, 2, 1>},
     {"T128_K4_B8_U2_loss", 128, (const void*)adds_cta_kernel<128, 4, 8, 2, 1>},
-#ifdef P6D_DEV
-    // 9-: shapes kept for experiments (tools/variants.py, P6D_ADDS_VARIANT)
-    {"T256_K8_B2_U1", 256, (const void*)adds_cta_kernel<256, 8, 2, 1, 0>},
-    {"T256_K8_B2_U2", 256, (const void*)adds_cta_kernel<256, 8, 2, 2, 0>},
-    {"T512_K4_B2_U1", 512, (const void*)adds_cta_kernel<512, 4, 2, 1, 0>},
-    {"T256_K4_B3_U2", 256, (const void*)adds_cta_kernel<256, 4, 3, 2, 0>},
-    {"T512_K4_B2_D", 512, (const void*)adds_cta_kernel<512, 4, 2, 0, 0>},
-#endif
 };
-constexpr int N_ADDS_VARIANTS = sizeof(g_adds_variants) / sizeof(g_adds_variants[0]);
-static_assert(N_ADDS_VARIANTS <= P6D_MAX_VARIANTS, "raise P6D_MAX_VARIANTS");
 
 static inline int size_class(int nmax) { return nmax <= 512 ? 0 : (nmax <= 1024 ? 1 : 2); }
 static const int kPtxasVariant[3] = {2, 1, 0};
@@ -473,7 +409,7 @@ static bool class_is_relaid(int cls) { return p6d_sched_state[16 + cls] == 't'; 
 // agree; on any difference the class falls back to the ptxas kernel for the rest of the process.
 //   0 = not checked yet, 1 = verified, 2 = rejected
 static std::atomic<int> g_relaid_state[64][3];
-static std::recursive_mutex g_config_mu;                // launch configuration + self-check (cold paths only)
+static std::mutex g_selfcheck_mu;                       // the self-check (cold path)
 
 static bool relaid_disabled_by_env() {
     static const bool off = [] {
@@ -488,10 +424,6 @@ static int selfcheck_class(const p6d_mesh_table* t, int cls, int64_t n_poses, in
 // Variant for this launch.  May run the one-time self-check (synchronous, ~1 ms + allocations).
 static int pick_variant(const p6d_mesh_table* t, bool loss, cudaStream_t st, int* vi_out) {
     const int cls = size_class(t->max_count);
-#ifdef P6D_DEV
-    static const int forced = [] { const char* e = getenv("P6D_ADDS_VARIANT"); return e ? atoi(e) : -1; }();
-    if (forced >= 0 && forced < N_ADDS_VARIANTS) { *vi_out = forced; return P6D_OK; }
-#endif
     if (loss) { *vi_out = kLossVariant[cls]; return P6D_OK; }
     *vi_out = kPtxasVariant[cls];
     if (!class_is_relaid(cls) || relaid_disabled_by_env()) return P6D_OK;
@@ -501,7 +433,7 @@ static int pick_variant(const p6d_mesh_table* t, bool loss, cudaStream_t st, int
         cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
         if (st && cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap != cudaStreamCaptureStatusNone)
             return P6D_OK;       // cannot synchronise inside a capture: this launch keeps ptxas' schedule
-        std::lock_guard<std::recursive_mutex> lock(g_config_mu);
+        std::lock_guard<std::mutex> lock(g_selfcheck_mu);
         sv = state.load(std::memory_order_acquire);
         if (sv == 0) {
             int64_t bad = 0;
@@ -559,6 +491,25 @@ int raise_dyn_smem(const void* fn, int device, size_t bytes) {
     return P6D_OK;
 }
 
+int ctas_per_sm(const void* fn, int threads, int device, size_t smem, int* per_sm) {
+    struct Shape { const void* fn; int device; size_t smem; int per_sm; };
+    static std::mutex mu;
+    static std::vector<Shape> known;
+    std::lock_guard<std::mutex> lock(mu);
+    auto it = std::find_if(known.begin(), known.end(),
+                           [&](const Shape& k) { return k.fn == fn && k.device == device && k.smem == smem; });
+    if (it == known.end()) {
+        // the occupancy query assumes the attribute already admits smem
+        int rc = raise_dyn_smem(fn, device, smem);
+        if (rc) return rc;
+        int occ = 0;
+        P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, threads, smem));
+        it = known.insert(known.end(), Shape{fn, device, smem, occ < 1 ? 1 : occ});
+    }
+    *per_sm = it->per_sm;
+    return P6D_OK;
+}
+
 int claim_counter(const p6d_mesh_table* t, cudaStream_t st, int** counter) {
     *counter = t->d_counters + (__atomic_fetch_add(&t->counter_idx, 1u, __ATOMIC_RELAXED) % P6D_NUM_COUNTERS);
     P6D_CUDA(cudaMemsetAsync(*counter, 0, sizeof(int), st));
@@ -579,13 +530,10 @@ static int adds_max_points_for(int smem_limit) {
     return lo;
 }
 
-// CTAs per SM of variant vi for this table; computed once per (table, variant), thread-safe
-static int configure_variant(const p6d_mesh_table* t, int vi, size_t smem, int* per_sm) {
-    int v = __atomic_load_n(&t->adds_per_sm[vi], __ATOMIC_ACQUIRE);
-    if (v > 0) { *per_sm = v; return P6D_OK; }
-    std::lock_guard<std::recursive_mutex> lock(g_config_mu);
+// the table's largest mesh fits the resident ADD-S kernel on its device
+static int check_resident_size(const p6d_mesh_table* t) {
     int limit = 0;
-    int rc = max_optin_smem(t->device, &limit);
+    const int rc = max_optin_smem(t->device, &limit);
     if (rc) return rc;
     if (!resident_fits(t, limit)) {
         set_error("largest mesh has %d points; the ADD-S kernel holds the mesh, the gt cloud and two "
@@ -593,13 +541,6 @@ static int configure_variant(const p6d_mesh_table* t, int vi, size_t smem, int* 
                   t->max_count, adds_max_points_for(limit));
         return P6D_ETOOBIG;
     }
-    const AddsVariant& var = g_adds_variants[vi];
-    if ((rc = raise_dyn_smem(var.fn, t->device, smem))) return rc;
-    int occ = 0;
-    P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, var.fn, var.threads, smem));
-    v = occ < 1 ? 1 : occ;
-    __atomic_store_n(&t->adds_per_sm[vi], v, __ATOMIC_RELEASE);
-    *per_sm = v;
     return P6D_OK;
 }
 
@@ -615,18 +556,12 @@ static int launch_resident(const p6d_mesh_table* t, const EvalArgs& args, int vi
     const size_t smem = adds_smem_bytes(t->max_count);
     const AddsVariant& var = g_adds_variants[vi];
     int per_sm = 0;
-    int rc = configure_variant(t, vi, smem, &per_sm);
+    int rc = check_resident_size(t);
+    if (rc == P6D_OK) rc = ctas_per_sm(var.fn, var.threads, t->device, smem, &per_sm);
     if (rc) return rc;
     int64_t grid = static_cast<int64_t>(t->sm_count) * per_sm;
     if (grid > args.B) grid = args.B;
     EvalArgs a2 = args;
-#ifdef P6D_DEV
-    {
-        // measurement knob (tools/variants.py): repeat the all-pairs scan to isolate its rate
-        static const int reps = [] { const char* e = getenv("P6D_DEBUG_SCAN_REPS"); const int r = e ? atoi(e) : 1; return r < 1 ? 1 : r; }();
-        a2.scan_reps = reps;
-    }
-#endif
     if ((rc = claim_counter(t, st, &a2.work_counter))) return rc;
     int nmax = t->max_count;
     void* kargs[] = {&a2, &nmax};
@@ -800,7 +735,7 @@ int p6d_adds_selfcheck(const p6d_mesh_table* table, int64_t n_poses, int64_t* mi
     if (!class_is_relaid(cls)) return P6D_OK;      // nothing re-laid in this build: nothing to compare
     DeviceGuard guard(table->device);
     if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    std::lock_guard<std::recursive_mutex> lock(g_config_mu);
+    std::lock_guard<std::mutex> lock(g_selfcheck_mu);
     const int rc = selfcheck_class(table, cls, n_poses, mismatches);
     if (rc) return rc;
     std::atomic<int>& state = g_relaid_state[table->device & 63][cls];
@@ -936,12 +871,16 @@ int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable) {
 // float4 / float2 / int4 loads in the kernels need their natural alignment
 static bool misaligned(const void* p, size_t a) { return p && (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
 
-// Argument checks of the device-buffer evaluation entries (messages prefixed with `fn`), then *a.  need_adds: the
-// entry computes ADD-S in any case (p6d_add_eval_pruned).
-static int eval_entry_args(const char* fn, bool need_adds, const p6d_mesh_table* table, const float* pq,
-                           const float* pt, const float* gq, const float* gt, const int64_t* obj, const int32_t* order,
-                           int64_t B, float* add, float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
-                           const p6d_accumulators* acc, EvalArgs* a) {
+// The three device-buffer evaluation entries: p6d_add_eval routes through launch_eval, the other two launch their
+// kernel directly.  Error messages are prefixed with the entry's name.
+enum EvalEntry { EVAL_ROUTED, EVAL_PRUNED, EVAL_STREAMED };
+
+static int eval_entry(EvalEntry which, const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                      const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add, float* adds,
+                      uint8_t* hit, uint8_t* valid, uint8_t* borderline, const p6d_accumulators* acc, void* stream) {
+    static const char* const names[] = {"p6d_add_eval", "p6d_add_eval_pruned", "p6d_add_eval_streamed"};
+    const char* fn = names[which];
+    const bool need_adds = which == EVAL_PRUNED;   // the pruned kernel computes ADD-S in any case
     if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || (need_adds && !adds) || !hit || !valid))) {
         set_error("%s: bad arguments", fn);
         return P6D_EINVAL;
@@ -956,12 +895,20 @@ static int eval_entry_args(const char* fn, bool need_adds, const p6d_mesh_table*
                   static_cast<long long>(B), INT32_MAX - (1 << 20));
         return P6D_EINVAL;
     }
-    *a = EvalArgs{};
-    fill_eval_args(table, *a);
-    a->pq = pq; a->pt = pt; a->gq = gq; a->gt = gt; a->obj = obj; a->order = order; a->B = B;
-    a->add = add; a->adds = adds; a->hit = hit; a->valid = valid; a->borderline = borderline;
-    if (acc) { a->acc = *acc; a->has_acc = 1; }
-    return P6D_OK;
+    if (B == 0) return P6D_OK;
+    EvalArgs a{};
+    fill_eval_args(table, a);
+    a.pq = pq; a.pt = pt; a.gq = gq; a.gt = gt; a.obj = obj; a.order = order; a.B = B;
+    a.add = add; a.adds = adds; a.hit = hit; a.valid = valid; a.borderline = borderline;
+    if (acc) { a.acc = *acc; a.has_acc = 1; }
+    DeviceGuard guard(table->device);
+    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
+    const cudaStream_t st = static_cast<cudaStream_t>(stream);
+    switch (which) {
+        case EVAL_PRUNED: return launch_eval_pruned(table, a, st);
+        case EVAL_STREAMED: return launch_eval_streamed(table, a, adds != nullptr, st);
+        default: return launch_eval(table, a, adds != nullptr, st, nullptr);
+    }
 }
 
 extern "C" {
@@ -970,39 +917,22 @@ int p6d_add_eval(const p6d_mesh_table* table, const float* pq, const float* pt, 
                  const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
                  float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                  const p6d_accumulators* acc, void* stream) {
-    EvalArgs a;
-    const int rc = eval_entry_args("p6d_add_eval", false, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid,
-                                   borderline, acc, &a);
-    if (rc != P6D_OK || B == 0) return rc;
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    return launch_eval(table, a, adds != nullptr, static_cast<cudaStream_t>(stream), nullptr);
+    return eval_entry(EVAL_ROUTED, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid, borderline, acc, stream);
 }
 
 int p6d_add_eval_pruned(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                         const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
                         float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                         const p6d_accumulators* acc, void* stream) {
-    EvalArgs a;
-    const int rc = eval_entry_args("p6d_add_eval_pruned", true, table, pq, pt, gq, gt, obj, order, B, add, adds, hit,
-                                   valid, borderline, acc, &a);
-    if (rc != P6D_OK || B == 0) return rc;
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    return launch_eval_pruned(table, a, static_cast<cudaStream_t>(stream));
+    return eval_entry(EVAL_PRUNED, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid, borderline, acc, stream);
 }
 
 int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                           const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
                           float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                           const p6d_accumulators* acc, void* stream) {
-    EvalArgs a;
-    const int rc = eval_entry_args("p6d_add_eval_streamed", false, table, pq, pt, gq, gt, obj, order, B, add, adds,
-                                   hit, valid, borderline, acc, &a);
-    if (rc != P6D_OK || B == 0) return rc;
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    return launch_eval_streamed(table, a, adds != nullptr, static_cast<cudaStream_t>(stream));
+    return eval_entry(EVAL_STREAMED, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid, borderline, acc,
+                      stream);
 }
 
 int64_t p6d_add_forward_workspace_bytes(const p6d_mesh_table* table, int64_t B) {
@@ -1119,37 +1049,6 @@ int p6d_add_eval_host(p6d_mesh_table* t, const float* pq, const float* pt, const
     if (acc_adds_sum) memcpy(acc_adds_sum, h + 24 * ns, 8 * ns);
     return P6D_OK;
 }
-
-#ifdef P6D_DEV
-int p6d_adds_timeline(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
-                      const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
-                      float* adds, uint8_t* hit, uint8_t* valid, uint64_t* timeline_host, int max_ctas,
-                      int* n_ctas) {
-    if (!table || B <= 0 || !timeline_host || !n_ctas || !adds) { set_error("p6d_adds_timeline: bad arguments"); return P6D_EINVAL; }
-    DeviceGuard guard(table->device);
-    if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
-    unsigned long long* d_tl = nullptr;
-    P6D_CUDA(cudaMalloc(&d_tl, sizeof(unsigned long long) * 4 * 4096));
-    P6D_CUDA(cudaMemset(d_tl, 0, sizeof(unsigned long long) * 4 * 4096));
-    EvalArgs a{};
-    fill_eval_args(table, a);
-    a.pq = pq; a.pt = pt; a.gq = gq; a.gt = gt; a.obj = obj; a.order = order; a.B = B;
-    a.add = add; a.adds = adds; a.hit = hit; a.valid = valid; a.timeline = d_tl;
-    int grid = 0;
-    int rc = launch_eval(table, a, true, nullptr, nullptr, &grid);
-    if (rc == P6D_OK) {
-        cudaError_t e = cudaDeviceSynchronize();
-        if (e != cudaSuccess) rc = cuda_fail(e, "cudaDeviceSynchronize");
-    }
-    if (rc == P6D_OK) {
-        const int n = grid < max_ctas ? grid : max_ctas;
-        cudaMemcpy(timeline_host, d_tl, sizeof(unsigned long long) * 4 * n, cudaMemcpyDeviceToHost);
-        *n_ctas = n;
-    }
-    cudaFree(d_tl);
-    return rc;
-}
-#endif
 
 int p6d_quat_to_mat(const float* q, int64_t B, float* R, int device, void* stream) {
     if (B < 0 || (B > 0 && (!q || !R))) { set_error("p6d_quat_to_mat: bad arguments"); return P6D_EINVAL; }

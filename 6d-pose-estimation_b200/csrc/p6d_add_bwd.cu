@@ -40,8 +40,7 @@ __global__ void __launch_bounds__(BWD_T) add_backward_kernel(BwdArgs a, int nmax
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int64_t b = blockIdx.x; b < a.B; b += gridDim.x) {
         const int64_t oid = a.obj[b];
-        const bool known = oid >= 0 && oid < a.n_slots && a.slots[oid].count > 0;
-        if (!known) {  // skipped sample: no gradient (add_loss.py:113)
+        if (!slot_known(oid, a.n_slots, a.slots)) {  // skipped sample: no gradient (add_loss.py:113)
             if (tid < 4) a.grad_q[4 * b + tid] = 0.0f;
             if (tid < 3) a.grad_t[3 * b + tid] = 0.0f;
             continue;

@@ -258,23 +258,12 @@ __global__ void __launch_bounds__(T, MINB) adds_pruned_kernel(EvalArgs a, Pruned
         const int64_t it = s_next;
         if (it >= a.B) break;
         const int64_t b = a.order ? a.order[it] : it;
-        if (tid < 4) s_pose[tid] = __ldg(a.pq + 4 * b + tid);
-        else if (tid < 8) s_pose[tid] = __ldg(a.gq + 4 * b + tid - 4);
-        else if (tid < 11) s_pose[tid] = __ldg(a.pt + 3 * b + tid - 8);
-        else if (tid < 14) s_pose[tid] = __ldg(a.gt + 3 * b + tid - 11);
-        else if (tid == 32) s_oid = a.obj[b];
+        load_pose(a, b, tid, s_pose, &s_oid);
         __syncthreads();  // (A) also: the previous pose's readers of shared memory are done
         if (tid == 64) s_next = atomicAdd(a.work_counter, 1);   // read after barriers (B) and (C)
         const long long oid = s_oid;
-        const bool known = oid >= 0 && oid < a.n_slots && a.slots[oid].count > 0;
-        if (!known) {  // CTA-uniform
-            if (tid == 0) {
-                a.add[b] = 0.0f;
-                a.adds[b] = 0.0f;
-                a.hit[b] = 0;
-                a.valid[b] = 0;
-                if (a.borderline) a.borderline[b] = 0;
-            }
+        if (!slot_known(oid, a.n_slots, a.slots)) {  // CTA-uniform
+            if (tid == 0) write_skipped(a, b, true);
             __syncthreads();
             continue;
         }
@@ -282,13 +271,7 @@ __global__ void __launch_bounds__(T, MINB) adds_pruned_kernel(EvalArgs a, Pruned
         const PrunedSlot ps = pa.pslots[oid];
         const int n = s.count, nb = ps.nb, np = PR_BLOCK * nb, nbp = (nb + 3) / 4 * 4;
         if (oid != staged_oid) {
-            if (tid == 0) {
-                fence_proxy_async();
-                const uint32_t bytes = static_cast<uint32_t>(ps.floats) * sizeof(float);
-                mbar_arrive_expect_tx(&s_bar, bytes);
-                tma_bulk_g2s(s_sorted, pa.sorted + ps.offset, bytes, &s_bar);
-            }
-            mbar_wait(&s_bar, phase);
+            stage_mesh(s_sorted, pa.sorted + ps.offset, ps.floats, &s_bar, phase, tid);
             phase ^= 1;
             staged_oid = oid;
         }
@@ -403,21 +386,8 @@ __global__ void __launch_bounds__(T, MINB) adds_pruned_kernel(EvalArgs a, Pruned
 
         // phase D: ordered means (ATen summation order) on warps 0 and 1, decision, outputs
         if (tid < 64) {
-            const float* src = tid < 32 ? s_dadd : s_dadds;
-            const float mean = aten_mean_warp([&](int e) { return src[e]; }, n, lane);
-            if (lane == 0) s_mean[tid >> 5] = mean;
-            asm volatile("bar.sync 1, 64;" ::: "memory");
-            if (tid == 0) {
-                const float add = s_mean[0], adds = s_mean[1];
-                const float eff = s.symmetric ? adds : add;
-                const bool is_hit = static_cast<double>(eff) < s.threshold;
-                a.add[b] = add;
-                a.adds[b] = adds;
-                a.hit[b] = is_hit ? 1 : 0;
-                a.valid[b] = 1;
-                if (a.borderline) a.borderline[b] = near_threshold(eff, s.threshold) ? 1 : 0;
-                accumulate(a, oid, is_hit, add, adds, true);
-            }
+            ordered_means(s_dadd, s_dadds, n, tid, lane, true, s_mean, [](const float* p) { return *p; });
+            if (tid == 0) write_pose(a, b, oid, s, s_mean[0], s_mean[1], true);
         }
         // barrier (A) of the next pose protects the shared arrays
     }
@@ -452,9 +422,6 @@ int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaSt
     }
     const int nb = ptab->max_nb > 0 ? ptab->max_nb : 1;
     const size_t smem = pruned_smem_bytes(table);
-    for (const void* fn : {(const void*)adds_pruned_kernel<256, 2>, (const void*)adds_pruned_kernel<256, 3>,
-                           (const void*)adds_pruned_kernel<256, 4>, (const void*)adds_pruned_kernel<128, 8>})
-        if ((rc = raise_dyn_smem(fn, table->device, smem))) return rc;
     EvalArgs a = args;
     if ((rc = claim_counter(table, st, &a.work_counter))) return rc;
     // the instantiation whose register budget matches what shared memory lets be resident (see the kernel's comment)
@@ -465,15 +432,12 @@ int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaSt
     int per_sm = 0;
     for (const Shape& sh : shapes) {
         if (sh.threads == 128 && nb > 16) continue;           // small CTAs for meshes of <= 512 points only
-        int occ = 0;
-        P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, sh.fn, sh.threads, smem));
-        if (occ >= sh.minb || &sh == &shapes[3]) {
+        if ((rc = ctas_per_sm(sh.fn, sh.threads, table->device, smem, &per_sm))) return rc;
+        if (per_sm >= sh.minb || &sh == &shapes[3]) {
             pick = &sh;
-            per_sm = occ;
             break;
         }
     }
-    if (per_sm < 1) per_sm = 1;
     int64_t grid = static_cast<int64_t>(table->sm_count) * per_sm;
     if (grid > a.B) grid = a.B;
     PrunedArgs pa{ptab->d_sorted, ptab->d_slots};

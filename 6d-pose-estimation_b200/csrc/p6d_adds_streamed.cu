@@ -22,7 +22,6 @@
 // The workspace (8 bytes per point and pose, plus tickets) is allocated stream-ordered on the caller's stream and
 // the batch is launched in chunks that keep it within 64 MB, so two streams never share a buffer.
 #include <algorithm>
-#include <atomic>
 
 #include "p6d_common.cuh"
 
@@ -72,22 +71,11 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
         const int pi = static_cast<int>(it / sa.nblk), j = static_cast<int>(it % sa.nblk);
         const int64_t idx = sa.first + pi;
         const int64_t b = a.order ? a.order[idx] : idx;
-        if (tid < 4) s_pose[tid] = __ldg(a.pq + 4 * b + tid);
-        else if (tid < 8) s_pose[tid] = __ldg(a.gq + 4 * b + tid - 4);
-        else if (tid < 11) s_pose[tid] = __ldg(a.pt + 3 * b + tid - 8);
-        else if (tid < 14) s_pose[tid] = __ldg(a.gt + 3 * b + tid - 11);
-        else if (tid == 32) s_oid = a.obj[b];
+        load_pose(a, b, tid, s_pose, &s_oid);
         __syncthreads();  // (B) also: every thread has read s_item
         const long long oid = s_oid;
-        const bool known = oid >= 0 && oid < a.n_slots && a.slots[oid].count > 0;
-        if (!known) {  // CTA-uniform; the first item of the pose writes its outputs
-            if (tid == 0 && j == 0) {
-                a.add[b] = 0.0f;
-                if (ADDS) a.adds[b] = 0.0f;
-                a.hit[b] = 0;
-                a.valid[b] = 0;
-                if (a.borderline) a.borderline[b] = 0;
-            }
+        if (!slot_known(oid, a.n_slots, a.slots)) {  // CTA-uniform; the first item of the pose writes its outputs
+            if (tid == 0 && j == 0) write_skipped(a, b, ADDS);
             continue;
         }
         const SlotInfo s = a.slots[oid];
@@ -206,22 +194,8 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
         if (!s_last) continue;
         __threadfence();
         if (tid < (ADDS ? 64 : 32)) {
-            const float* src = tid < 32 ? row_add : row_adds;
-            const float mean = aten_mean_warp([&](int e) { return __ldcg(src + e); }, n, lane);
-            if (lane == 0) s_mean[tid >> 5] = mean;
-            if (ADDS) asm volatile("bar.sync 1, 64;" ::: "memory");
-            else __syncwarp();
-            if (tid == 0) {
-                const float add = s_mean[0], adds = ADDS ? s_mean[1] : 0.0f;
-                const float eff = (ADDS && s.symmetric) ? adds : add;   // without ADD-S, symmetric ids decide on ADD
-                const bool is_hit = static_cast<double>(eff) < s.threshold;
-                a.add[b] = add;
-                if (ADDS) a.adds[b] = adds;
-                a.hit[b] = is_hit ? 1 : 0;
-                a.valid[b] = 1;
-                if (a.borderline) a.borderline[b] = near_threshold(eff, s.threshold) ? 1 : 0;
-                accumulate(a, oid, is_hit, add, adds, ADDS);
-            }
+            ordered_means(row_add, row_adds, n, tid, lane, ADDS, s_mean, [](const float* p) { return __ldcg(p); });
+            if (tid == 0) write_pose(a, b, oid, s, s_mean[0], ADDS ? s_mean[1] : 0.0f, ADDS);
         }
     }
 }
@@ -239,7 +213,6 @@ static const StShape kStShapes[2][3] = {
      {(const void*)adds_streamed_kernel<4, 4, true>, 4},
      {(const void*)adds_streamed_kernel<2, 4, true>, 2}},
 };
-static std::atomic<int> g_st_per_sm[64][2][3];   // CTAs per SM (0 = not computed yet)
 
 int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st) {
     if (t->max_count > ST_MAX_POINTS) {
@@ -262,13 +235,9 @@ int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool wan
     const int ai = want_adds ? 1 : 0;
     int pick = 2, per_sm_pick = 1;
     for (int si = 0; si < 3; ++si) {
-        std::atomic<int>& cache = g_st_per_sm[t->device & 63][ai][si];
-        int per_sm = cache.load(std::memory_order_relaxed);
-        if (per_sm == 0) {
-            P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kStShapes[ai][si].fn, ST_T, 0));
-            per_sm = std::max(per_sm, 1);
-            cache.store(per_sm, std::memory_order_relaxed);
-        }
+        int per_sm = 0;
+        int rc = ctas_per_sm(kStShapes[ai][si].fn, ST_T, t->device, 0, &per_sm);
+        if (rc) return rc;
         const int P = ST_T * kStShapes[ai][si].k;
         const int64_t items = bc * ((nmax + P - 1) / P);
         if (items >= 2 * static_cast<int64_t>(t->sm_count) * per_sm || si == 2) {

@@ -8,8 +8,6 @@
 // Elementwise, HBM/latency-bound: one thread per row, K read as scalars (4 of the 9
 // entries), everything else coalesced.  Operation order is the reference's:
 // ((u - cx) * z) / fx with an IEEE division.
-#include <map>
-#include <mutex>
 
 #include "p6d_common.cuh"
 
@@ -357,23 +355,12 @@ __global__ void __launch_bounds__(CAM_T) project_points_kernel(const double* __r
 // Grid of a grid-stride kernel: one thread per row up to what is RESIDENT at once.  Every block of a grid-stride
 // loop runs the same number of trips, so blocks beyond the resident set form a second, thinly occupied wave that
 // takes as long as the first (the 40-register shared-K pinhole kernel fits 6 blocks per SM: a fixed cap of 8 per
-// SM ran 1.33 waves and reached 72 % of HBM).  Occupancy is asked once per kernel.
+// SM ran 1.33 waves and reached 72 % of HBM).
 template <class Kernel>
 static int grid_for(Kernel kernel, int64_t B, int device, unsigned* grid) {
-    static std::mutex mu;
-    static std::map<const void*, int> cache;        // kernels of one signature share this instantiation: key by address
     int per_sm = 0;
-    {
-        std::lock_guard<std::mutex> lock(mu);
-        auto it = cache.find(reinterpret_cast<const void*>(kernel));
-        if (it != cache.end()) per_sm = it->second;
-    }
-    if (per_sm == 0) {
-        P6D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, CAM_T, 0));
-        if (per_sm < 1) per_sm = 1;
-        std::lock_guard<std::mutex> lock(mu);
-        cache[reinterpret_cast<const void*>(kernel)] = per_sm;
-    }
+    int rc = ctas_per_sm(reinterpret_cast<const void*>(kernel), CAM_T, device, 0, &per_sm);
+    if (rc) return rc;
     int sms = 0;
     P6D_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
     int64_t blocks = (B + CAM_T - 1) / CAM_T;

@@ -205,17 +205,6 @@ int p6d_add_backward(const p6d_mesh_table* table, const float* pq, const float* 
                      const float* gt, const int64_t* obj, int64_t B, const float* grad_out,
                      const int32_t* count, float inv_count, float* grad_q, float* grad_t, void* stream);
 
-#ifdef P6D_DEV   /* development build only (make -C csrc dev) */
-/* Measurement helper: runs the ADD-S kernel once (device buffers, legacy stream, synchronous)
- * and returns, per CTA, {smid, globaltimer start, globaltimer end, poses processed} so the
- * load balance of the persistent grid can be inspected.  timeline_host holds 4*max_ctas
- * uint64; n_ctas receives the grid size (<= 4096). */
-int p6d_adds_timeline(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
-                      const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
-                      float* adds, uint8_t* hit, uint8_t* valid, uint64_t* timeline_host, int max_ctas,
-                      int* n_ctas);
-#endif
-
 /* Quaternion -> rotation matrix, ADDLoss._quat_to_mat (models/add_loss.py:203-215). */
 int p6d_quat_to_mat(const float* q, int64_t B, float* R, int device, void* stream);
 

@@ -7,8 +7,7 @@ output hash is compared with the baseline's.
 
   python tools/sched_search.py UNPATCHED.so KERNEL CLASS N_POINTS POSES BUDGET_SECONDS [policy|plan.json] [yield]
 UNPATCHED.so is the PRODUCT library as ptxas made it (make NOSCHED=1 TARGET=...): the plan is only valid
-for the loop it was measured on (sass_sched.fingerprint), and the development build compiles another
-loop.  CLASS = 0 / 1 / 2 (N <= 512, <= 1024, larger): the letter of p6d_sched_state the candidate sets,
+for the loop it was measured on (sass_sched.fingerprint).  CLASS = 0 / 1 / 2 (N <= 512, <= 1024, larger): the letter of p6d_sched_state the candidate sets,
 which makes the library use the re-laid kernel of that class -- after its own run-time self-check
 against the ptxas-scheduled kernel, so a candidate that computes anything else is rejected twice.
 A plan.json measured on another instruction order of the loop is used as a starting point by slot
