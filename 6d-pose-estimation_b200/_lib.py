@@ -33,6 +33,7 @@ EXPORTS = (
     "p6d_adds_selfcheck", "p6d_selftest_sqrt2", "p6d_add_eval", "p6d_add_eval_pruned", "p6d_mesh_table_set_pruning", "p6d_add_eval_streamed",
     "p6d_mesh_table_set_large_meshes", "p6d_add_eval_host",
     "p6d_add_forward_workspace_bytes", "p6d_add_forward", "p6d_add_backward",
+    "p6d_mesh_table_set_large_mesh_loss", "p6d_add_forward_streamed", "p6d_add_backward_streamed",
     "p6d_quat_to_mat", "p6d_pose_loss_workspace_bytes", "p6d_pose_loss_fwd_bwd",
     "p6d_pose_loss_pinhole_fwd_bwd", "p6d_pinhole_fwd", "p6d_pinhole_bwd", "p6d_depth_backproject",
     "p6d_depth_crop_backproject", "p6d_detection_backproject", "p6d_project_points", "p6d_synth_poses", "p6d_sweep_run",
@@ -93,6 +94,8 @@ def lib() -> C.CDLL:
     L.p6d_add_forward_workspace_bytes.argtypes = [vp, i64]
     L.p6d_add_forward_workspace_bytes.restype = i64
     L.p6d_add_forward.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp, vp, vp, vp]
+    L.p6d_add_forward_streamed.argtypes = L.p6d_add_forward.argtypes
+    L.p6d_mesh_table_set_large_mesh_loss.argtypes = [vp, i32]
     u64 = C.c_uint64
     L.p6d_synth_poses.argtypes = [u64, i32, i32, i64, i64, f32, f32, i32, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                   i32, vp]
@@ -112,6 +115,7 @@ def lib() -> C.CDLL:
     L.p6d_detection_backproject.argtypes = [vp, i32, i32, vp, i64, vp, i32, vp, vp, vp, vp, i32, vp]
     L.p6d_project_points.argtypes = [vp, i32, vp, i32, vp, vp, i64, vp, i32, vp]
     L.p6d_add_backward.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp, vp, f32, vp, vp, vp]
+    L.p6d_add_backward_streamed.argtypes = L.p6d_add_backward.argtypes
     missing = [n for n in EXPORTS if not hasattr(L, n)]
     if missing:
         raise P6DError(f"{SO_PATH} is stale: missing symbols {missing}; rebuild it")
@@ -236,6 +240,14 @@ class MeshTable:
         check(lib().p6d_mesh_table_set_large_meshes(self.handle, 1 if enable else 0))
         return self
 
+    def set_large_mesh_loss(self, enable=True):
+        """Opt in to (or out of) the streamed loss-form and gradient kernels for this table: the same loss bits
+        as the resident loss form, taken by forward_loss / add_backward only when the largest mesh is beyond the
+        resident kernels' shared-memory limit (up to 32,768 points); independent of set_large_meshes; see
+        include/p6d.h."""
+        check(lib().p6d_mesh_table_set_large_mesh_loss(self.handle, 1 if enable else 0))
+        return self
+
     # -- device-buffer evaluation ---------------------------------------------------
     def evaluate_packed(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False):
         """Launch the evaluation kernels on the current stream and return the ONE buffer behind the
@@ -283,17 +295,19 @@ class MeshTable:
         torch.cuda.current_stream(self.device).synchronize()
         return host.numpy()
 
-    def forward_loss(self, pq, pt, gq, gt, obj):
+    def forward_loss(self, pq, pt, gq, gt, obj, streamed=False):
         """ADDLoss.forward value: one launch, no host synchronisation.  Returns (loss [1] f32,
-        count [1] i32) device tensors."""
+        count [1] i32) device tensors.  streamed: always the streamed loss form (p6d_add_forward_streamed)
+        instead of the table's choice."""
         B = obj.shape[0]
         dev = self.device
         L = lib()
         ws = torch.empty(int(L.p6d_add_forward_workspace_bytes(self.handle, B)) + 16, dtype=torch.uint8, device=dev)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         count = torch.empty(1, dtype=torch.int32, device=dev)
-        check(L.p6d_add_forward(self.handle, ptr(pq), ptr(pt), ptr(gq), ptr(gt), ptr(obj), B, ptr(loss), ptr(count),
-                                ptr(ws), stream_ptr(dev)))
+        entry = L.p6d_add_forward_streamed if streamed else L.p6d_add_forward
+        check(entry(self.handle, ptr(pq), ptr(pt), ptr(gq), ptr(gt), ptr(obj), B, ptr(loss), ptr(count), ptr(ws),
+                    stream_ptr(dev)))
         return loss, count
 
     def schedule_state(self) -> dict:
@@ -338,15 +352,17 @@ class MeshTable:
                 "d2h_bytes": (B * (4 + (4 if want_adds else 0) + 3) if per_pose else 0) + 32 * ns}
 
 
-def add_backward(saved, grad_out):
+def add_backward(saved, grad_out, streamed=False):
     """Gradients of ADDLoss.forward w.r.t. (pred_r, pred_t) through p6d_add_backward; the number of
-    valid samples stays on the device (written by p6d_add_forward)."""
+    valid samples stays on the device (written by p6d_add_forward).  streamed: always the streamed
+    backward (p6d_add_backward_streamed) instead of the table's choice."""
     pq, pt, gq, gt, obj, count, table, dev = saved
     go = grad_out.detach().to(dev, torch.float32).reshape(1).contiguous()
     gq_out = torch.empty_like(pq)
     gt_out = torch.empty_like(pt)
-    check(lib().p6d_add_backward(table.handle, ptr(pq), ptr(pt), ptr(gq), ptr(gt), ptr(obj), obj.shape[0], ptr(go),
-                                 ptr(count), 0.0, ptr(gq_out), ptr(gt_out), stream_ptr(dev)))
+    entry = lib().p6d_add_backward_streamed if streamed else lib().p6d_add_backward
+    check(entry(table.handle, ptr(pq), ptr(pt), ptr(gq), ptr(gt), ptr(obj), obj.shape[0], ptr(go), ptr(count), 0.0,
+                ptr(gq_out), ptr(gt_out), stream_ptr(dev)))
     return gq_out, gt_out
 
 

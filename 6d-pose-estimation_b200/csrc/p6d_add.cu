@@ -127,68 +127,6 @@ __device__ __forceinline__ void scan_deferred(const float4* __restrict__ p, cons
     }
 }
 
-// Loss form (ADDLoss.forward, models/add_loss.py:118-150), run by the last CTA to finish: groups in
-// first-appearance order; per group the float32 ATen sum of its samples' values (index order) is
-// added to the running total; total / count.  ws: [0] ticket, [1..1+n_slots) first valid index per
-// object, then B floats of scratch for the compacted group.
-template <int T>
-__device__ void loss_finalize(const EvalArgs& a, int tid) {
-    __shared__ int s_warp_tot[T / 32];
-    __shared__ int s_pick[2];
-    const int lane = tid & 31, warp = tid >> 5;
-    int32_t* first = a.loss_ws + 1;
-    float* scratch = reinterpret_cast<float*>(a.loss_ws + 1 + a.n_slots);
-    const int B = static_cast<int>(a.B);
-    for (int s = tid; s < a.n_slots; s += T) first[s] = INT32_MAX;
-    __syncthreads();
-    for (int i = tid; i < B; i += T)
-        if (__ldcg(a.valid + i)) atomicMin(first + a.obj[i], i);
-    __syncthreads();
-    float total = 0.0f;
-    int count = 0, prev = -1;
-    for (;;) {
-        // next group: the object whose first sample comes next
-        if (tid == 0) { s_pick[0] = INT32_MAX; s_pick[1] = -1; }
-        __syncthreads();
-        int best = INT32_MAX;
-        for (int s = tid; s < a.n_slots; s += T) {
-            const int f = first[s];
-            if (f > prev && f < best) best = f;
-        }
-        if (best != INT32_MAX) atomicMin(&s_pick[0], best);
-        __syncthreads();
-        const int head = s_pick[0];
-        if (head == INT32_MAX) break;     // CTA-uniform
-        const int64_t oid = a.obj[head];
-        // compact the group's values in index order
-        int n = 0;
-        for (int base = 0; base < B; base += T) {
-            const int i = base + tid;
-            const bool mine = i < B && __ldcg(a.valid + i) && a.obj[i] == oid;
-            const unsigned m = __ballot_sync(0xffffffffu, mine);
-            if (lane == 0) s_warp_tot[warp] = __popc(m);
-            __syncthreads();
-            int off = n;
-            for (int w = 0; w < warp; ++w) off += s_warp_tot[w];
-            if (mine) scratch[off + __popc(m & ((1u << lane) - 1u))] = __ldcg(a.sample + i);
-            for (int w = 0; w < T / 32; ++w) n += s_warp_tot[w];
-            __syncthreads();
-        }
-        if (warp == 0) {
-            const float gs = aten_sum_warp([&](int e) { return scratch[e]; }, n, lane);
-            total = __fadd_rn(total, gs);     // lanes of warp 0 agree; other warps do not use it
-        }
-        count += n;
-        prev = head;
-        __syncthreads();
-    }
-    if (tid == 0) {
-        a.loss_out[0] = count > 0 ? __fdiv_rn(total, static_cast<float>(count)) : 0.0f;
-        a.count_out[0] = count;
-        a.loss_ws[0] = 0;                     // ticket left zeroed for the next call
-    }
-}
-
 // T threads per CTA, K pred points per thread, MINB CTAs per SM, U gt quads per loop trip
 // (U == 0: one quad per trip with software-pipelined minima, see scan_deferred);
 // LOSS = 1: the instantiation behind p6d_add_forward (per-sample value + grouped sum)
@@ -576,7 +514,9 @@ constexpr int PR_MIN_POINTS = 128;
 
 // Every evaluation call (p6d_add_eval, p6d_add_eval_host, p6d_add_forward, p6d_sweep_run) picks its kernel here,
 // and only here:
-//   * a forced variant (the self-check) or the loss form: the resident ADD-S kernel (b), pick_variant's variant;
+//   * a forced variant (the self-check): the resident ADD-S kernel (b) in that variant;
+//   * the loss form (p6d_add_forward): the streamed kernel's loss form if the table's large-mesh loss switch is on
+//     and the largest mesh is beyond the resident kernel's shared memory, the resident loss form otherwise;
 //   * without ADD-S: the ADD-only kernel (a); beyond its shared memory, the streamed kernel if the table's large-mesh
 //     switch is on;
 //   * pruning switch on, a block structure, a largest mesh of >= PR_MIN_POINTS that fits: the pruned kernel;
@@ -593,9 +533,16 @@ int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, c
         return P6D_EINVAL;
     }
     int rc = P6D_OK, vi = force_variant;
-    if (vi >= 0 || args.sample) {
-        if (vi < 0) rc = pick_variant(t, true, st, &vi);
-        if (rc == P6D_OK) rc = launch_resident(t, args, vi, st, grid_out);
+    if (vi >= 0) {
+        rc = launch_resident(t, args, vi, st, grid_out);
+    } else if (args.sample) {
+        const bool large = t->large_mesh_loss.load(std::memory_order_relaxed);
+        int limit = 0;
+        if (large && (rc = max_optin_smem(t->device, &limit))) return rc;
+        if (large && !resident_fits(t, limit))
+            rc = launch_eval_streamed(t, args, true, st);
+        else if ((rc = pick_variant(t, true, st, &vi)) == P6D_OK)
+            rc = launch_resident(t, args, vi, st, grid_out);
     } else {
         const bool large = t->large_meshes.load(std::memory_order_relaxed);
         const bool prune = want_adds && t->pruned && t->pruning.load(std::memory_order_relaxed) &&
@@ -866,6 +813,12 @@ int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable) {
     return P6D_OK;
 }
 
+int p6d_mesh_table_set_large_mesh_loss(p6d_mesh_table* table, int enable) {
+    if (!table) { set_error("p6d_mesh_table_set_large_mesh_loss: table is NULL"); return P6D_EINVAL; }
+    table->large_mesh_loss.store(enable != 0, std::memory_order_relaxed);
+    return P6D_OK;
+}
+
 }  // extern "C"
 
 // float4 / float2 / int4 loads in the kernels need their natural alignment
@@ -941,14 +894,19 @@ int64_t p6d_add_forward_workspace_bytes(const p6d_mesh_table* table, int64_t B) 
     return static_cast<int64_t>(sizeof(int32_t)) * (1 + table->n_slots) + 16 * B + 2 * B + 64;
 }
 
-int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
-                    const float* gt, const int64_t* obj, int64_t B, float* loss, int32_t* count,
-                    void* workspace, void* stream) {
+}  // extern "C"
+
+// p6d_add_forward routes through launch_eval; p6d_add_forward_streamed always takes the streamed kernel's loss form.
+static int forward_entry(bool streamed, const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                         const float* gt, const int64_t* obj, int64_t B, float* loss, int32_t* count, void* workspace,
+                         void* stream) {
+    const char* fn = streamed ? "p6d_add_forward_streamed" : "p6d_add_forward";
     if (!table || B < 0 || !loss || !count || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !workspace))) {
-        set_error("p6d_add_forward: bad arguments");
+        set_error("%s: bad arguments", fn);
         return P6D_EINVAL;
     }
-    if (misaligned(workspace, 16)) { set_error("p6d_add_forward: workspace must be 16-byte aligned"); return P6D_EINVAL; }
+    if (misaligned(workspace, 16)) { set_error("%s: workspace must be 16-byte aligned", fn); return P6D_EINVAL; }
+    if (streamed && check_streamed_size(table)) return P6D_ETOOBIG;
     DeviceGuard guard(table->device);
     if (!guard.ok) return cuda_fail(cudaGetLastError(), "cudaSetDevice");
     cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -957,7 +915,7 @@ int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* p
         P6D_CUDA(cudaMemsetAsync(count, 0, sizeof(int32_t), st));
         return P6D_OK;
     }
-    if (B > INT32_MAX / 2) { set_error("p6d_add_forward: batch too large"); return P6D_EINVAL; }
+    if (B > INT32_MAX / 2) { set_error("%s: batch too large", fn); return P6D_EINVAL; }
     char* w = static_cast<char*>(workspace);
     const size_t nB = static_cast<size_t>(B);
     EvalArgs a{};
@@ -972,7 +930,21 @@ int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* p
     a.valid = reinterpret_cast<uint8_t*>(w + off);
     a.loss_out = loss; a.count_out = count;
     P6D_CUDA(cudaMemsetAsync(a.loss_ws, 0, sizeof(int32_t), st));
-    return launch_eval(table, a, true, st, nullptr);
+    return streamed ? launch_eval_streamed(table, a, true, st) : launch_eval(table, a, true, st, nullptr);
+}
+
+extern "C" {
+
+int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                    const float* gt, const int64_t* obj, int64_t B, float* loss, int32_t* count,
+                    void* workspace, void* stream) {
+    return forward_entry(false, table, pq, pt, gq, gt, obj, B, loss, count, workspace, stream);
+}
+
+int p6d_add_forward_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                             const float* gt, const int64_t* obj, int64_t B, float* loss, int32_t* count,
+                             void* workspace, void* stream) {
+    return forward_entry(true, table, pq, pt, gq, gt, obj, B, loss, count, workspace, stream);
 }
 
 static int ensure_staging(p6d_mesh_table* t, size_t dev_bytes, size_t pin_bytes) {

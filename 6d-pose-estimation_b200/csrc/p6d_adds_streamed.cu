@@ -21,6 +21,11 @@
 //                phase D of adds_cta_kernel.
 // The workspace (8 bytes per point and pose, plus tickets) is allocated stream-ordered on the caller's stream and
 // the batch is launched in chunks that keep it within 64 MB, so two streams never share a buffer.
+//
+// Loss form (LOSS, ADDLoss.forward behind p6d_add_forward): transforms with the batched matmul's rounding
+// (s.xform_bmm), scans the gt tiles only for symmetric samples (the reference takes ADD for the others; the branch is
+// uniform per item), and the last item of a pose stores the per-sample value.  No launch sees the whole batch once
+// it is chunked, so the grouped sum (loss_finalize) runs as one single-CTA launch after the last chunk.
 #include <algorithm>
 
 #include "p6d_common.cuh"
@@ -30,7 +35,6 @@ namespace p6d {
 constexpr int ST_T = 256;                  // threads per CTA
 constexpr int ST_G = 1024;                 // gt points per tile (multiple of 8)
 constexpr int ST_STAGES = 2;               // TMA ring depth
-constexpr int ST_MAX_POINTS = 32768;       // see the refusal message in launch_eval_streamed
 constexpr size_t ST_WS_BYTES = size_t(64) << 20;
 
 struct StreamArgs {
@@ -43,8 +47,10 @@ struct StreamArgs {
     float* rows;        // [nposes][2][stride]: ADD row, ADD-S row
 };
 
-template <int K, int MINB, bool ADDS>
+// LOSS: an optional fourth argument, true for the loss form; the evaluation instantiations leave it out
+template <int K, int MINB, bool ADDS, bool... LOSS_>
 __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, StreamArgs sa) {
+    constexpr bool LOSS = (false || ... || LOSS_);
     constexpr int P = ST_T * K;
     __shared__ __align__(128) float s_raw[ST_STAGES][3 * ST_G];   // TMA destination: x | y | z of one tile
     __shared__ __align__(128) float s_quad[3 * ST_G];              // transformed tile as quads (48 B per 4 points)
@@ -75,11 +81,12 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
         __syncthreads();  // (B) also: every thread has read s_item
         const long long oid = s_oid;
         if (!slot_known(oid, a.n_slots, a.slots)) {  // CTA-uniform; the first item of the pose writes its outputs
-            if (tid == 0 && j == 0) write_skipped(a, b, ADDS);
+            if (tid == 0 && j == 0) write_skipped<LOSS>(a, b, ADDS);
             continue;
         }
         const SlotInfo s = a.slots[oid];
-        const int n = s.count, np = s.padded, mode = s.xform_mode;
+        const int n = s.count, np = s.padded, mode = LOSS ? s.xform_bmm : s.xform_mode;
+        const bool scan = ADDS && (!LOSS || s.symmetric);   // CTA-uniform
         if (j * P >= n) continue;  // beyond this pose's mesh: not counted in its ticket
         const int items = (n + P - 1) / P;
         const float* msh = a.soa + s.soa_offset;
@@ -97,7 +104,7 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
                 tp[k] = s_pose[8 + k];
                 tg[k] = s_pose[11 + k];
             }
-            if (ADDS && tid == 0) {
+            if (scan && tid == 0) {
 #pragma unroll
                 for (int k = 0; k < 9; ++k) s_rg[k] = Rg[k];
 #pragma unroll
@@ -118,7 +125,7 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
             }
         }
 
-        if (ADDS) {
+        if (scan) {
             const int ntiles = (n + ST_G - 1) / ST_G;
             auto issue = [&](int t) {  // one elected thread: tile t into its ring slot
                 const int st = t % ST_STAGES;
@@ -193,36 +200,49 @@ __global__ void __launch_bounds__(ST_T, MINB) adds_streamed_kernel(EvalArgs a, S
         __syncthreads();
         if (!s_last) continue;
         __threadfence();
-        if (tid < (ADDS ? 64 : 32)) {
-            ordered_means(row_add, row_adds, n, tid, lane, ADDS, s_mean, [](const float* p) { return __ldcg(p); });
-            if (tid == 0) write_pose(a, b, oid, s, s_mean[0], ADDS ? s_mean[1] : 0.0f, ADDS);
+        if (tid < (scan ? 64 : 32)) {
+            ordered_means(row_add, row_adds, n, tid, lane, scan, s_mean, [](const float* p) { return __ldcg(p); });
+            if (tid == 0) write_pose<LOSS>(a, b, oid, s, s_mean[0], scan ? s_mean[1] : 0.0f, scan);
         }
     }
+}
+
+template <int T>
+__global__ void __launch_bounds__(T) loss_finalize_kernel(EvalArgs a) {
+    loss_finalize<T>(a, threadIdx.x);
 }
 
 struct StShape {
     const void* fn;
     int k;
 };
-// per ADD-S flag, widest first
-static const StShape kStShapes[2][3] = {
+// ADD only, ADD-S, loss form; widest first
+static const StShape kStShapes[3][3] = {
     {{(const void*)adds_streamed_kernel<8, 2, false>, 8},
      {(const void*)adds_streamed_kernel<4, 4, false>, 4},
      {(const void*)adds_streamed_kernel<2, 4, false>, 2}},
     {{(const void*)adds_streamed_kernel<8, 2, true>, 8},
      {(const void*)adds_streamed_kernel<4, 4, true>, 4},
      {(const void*)adds_streamed_kernel<2, 4, true>, 2}},
+    {{(const void*)adds_streamed_kernel<8, 2, true, true>, 8},
+     {(const void*)adds_streamed_kernel<4, 4, true, true>, 4},
+     {(const void*)adds_streamed_kernel<2, 4, true, true>, 2}},
 };
 
+int check_streamed_size(const p6d_mesh_table* t) {
+    if (t->max_count <= ST_MAX_POINTS) return P6D_OK;
+    set_error("largest mesh has %d points; the streamed ADD/ADD-S kernel accepts at most %d points: above that, "
+              "torch's CPU Tensor.mean() splits a row across threads, so the reference's own result depends on "
+              "the caller's thread count and there is no single result to reproduce",
+              t->max_count, ST_MAX_POINTS);
+    return P6D_ETOOBIG;
+}
+
 int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, cudaStream_t st) {
-    if (t->max_count > ST_MAX_POINTS) {
-        set_error("largest mesh has %d points; the streamed ADD/ADD-S kernel accepts at most %d points: above that, "
-                  "torch's CPU Tensor.mean() splits a row across threads, so the reference's own result depends on "
-                  "the caller's thread count and there is no single result to reproduce",
-                  t->max_count, ST_MAX_POINTS);
-        return P6D_ETOOBIG;
-    }
+    int rc = check_streamed_size(t);
+    if (rc) return rc;
     if (args.B == 0) return P6D_OK;
+    const bool loss = args.sample != nullptr;
     const int nmax = t->max_count > 0 ? t->max_count : 1;
     const int stride = (nmax + 3) / 4 * 4;
     const size_t per_pose = 2 * sizeof(float) * static_cast<size_t>(stride) + sizeof(int);
@@ -232,12 +252,11 @@ int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool wan
     const size_t ws_bytes = head + 2 * sizeof(float) * static_cast<size_t>(stride) * static_cast<size_t>(bc);
 
     // the widest shape whose items fill the device at least twice; the narrowest otherwise
-    const int ai = want_adds ? 1 : 0;
+    const int ai = loss ? 2 : (want_adds ? 1 : 0);
     int pick = 2, per_sm_pick = 1;
     for (int si = 0; si < 3; ++si) {
         int per_sm = 0;
-        int rc = ctas_per_sm(kStShapes[ai][si].fn, ST_T, t->device, 0, &per_sm);
-        if (rc) return rc;
+        if ((rc = ctas_per_sm(kStShapes[ai][si].fn, ST_T, t->device, 0, &per_sm))) return rc;
         const int P = ST_T * kStShapes[ai][si].k;
         const int64_t items = bc * ((nmax + P - 1) / P);
         if (items >= 2 * static_cast<int64_t>(t->sm_count) * per_sm || si == 2) {
@@ -252,7 +271,6 @@ int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool wan
 
     char* ws = nullptr;
     P6D_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_bytes, st));
-    int rc = P6D_OK;
     for (int64_t c0 = 0; c0 < args.B && rc == P6D_OK; c0 += bc) {
         const int64_t nc = std::min<int64_t>(bc, args.B - c0);
         StreamArgs sa;
@@ -272,6 +290,13 @@ int launch_eval_streamed(const p6d_mesh_table* t, const EvalArgs& args, bool wan
         e = cudaLaunchKernel(shape.fn, dim3(static_cast<unsigned>(grid)), dim3(ST_T), kargs, 0, st);
         if (e == cudaSuccess) e = cudaGetLastError();
         if (e != cudaSuccess) rc = cuda_fail(e, "cudaLaunchKernel(adds_streamed_kernel)");
+    }
+    if (loss && rc == P6D_OK) {   // every chunk has stored its per-sample values: the grouped sum
+        EvalArgs a = args;
+        void* kargs[] = {&a};
+        cudaError_t e = cudaLaunchKernel((const void*)loss_finalize_kernel<ST_T>, dim3(1), dim3(ST_T), kargs, 0, st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) rc = cuda_fail(e, "cudaLaunchKernel(loss_finalize_kernel)");
     }
     const cudaError_t ef = cudaFreeAsync(ws, st);
     if (rc == P6D_OK && ef != cudaSuccess) rc = cuda_fail(ef, "cudaFreeAsync(streamed workspace)");

@@ -77,6 +77,7 @@ class ADDLoss(nn.Module):
         self._table_key = None
         self._table_pruning = False
         self._table_large = False
+        self._table_large_loss = False
         # optional callable(indices, pred_r, pred_t, gt_r, gt_t, obj_ids) -> 0/1 per index, consulted by
         # eval_metrics for decisions flagged `borderline`; None (default): the kernel's decision stands
         self.borderline_resolver = None
@@ -84,8 +85,12 @@ class ADDLoss(nn.Module):
         # all-pairs kernel is kept below that) -- not part of the reference surface, default off
         self.exact_pruning = False
         # opt-in: meshes beyond shared memory (up to 32,768 points) through the streamed kernel in eval_metrics /
-        # eval_poses (same bits; forward keeps its limit) -- not part of the reference surface, default off
+        # eval_poses (same bits; evaluation only) -- not part of the reference surface, default off
         self.large_meshes = False
+        # opt-in: meshes beyond shared memory (up to 32,768 points) through the streamed loss-form and gradient
+        # kernels in forward / train_loss and loss.backward() (same loss bits; the resident kernels wherever they
+        # run) -- not part of the reference surface, default off
+        self.large_mesh_loss = False
         self._load_models(model_dir)
 
     # ------------------------------------------------------------------ loading
@@ -149,12 +154,16 @@ class ADDLoss(nn.Module):
             self._table_key = key
             self._table_pruning = False
             self._table_large = False
+            self._table_large_loss = False
         if bool(self.exact_pruning) != self._table_pruning:
             self._table.set_pruning(bool(self.exact_pruning))
             self._table_pruning = bool(self.exact_pruning)
         if bool(self.large_meshes) != self._table_large:
             self._table.set_large_meshes(bool(self.large_meshes))
             self._table_large = bool(self.large_meshes)
+        if bool(self.large_mesh_loss) != self._table_large_loss:
+            self._table.set_large_mesh_loss(bool(self.large_mesh_loss))
+            self._table_large_loss = bool(self.large_mesh_loss)
         return self._table
 
     def _prepare(self, pred_r, pred_t, gt_r, gt_t, obj_ids, sort=True):

@@ -153,8 +153,9 @@ int p6d_add_eval_pruned(const p6d_mesh_table* table, const float* pq, const floa
  *                                    ADD-only outputs (symmetric ids then decide on ADD)
  *   p6d_mesh_table_set_large_meshes  per-table switch (default off): p6d_add_eval, p6d_add_eval_host and p6d_sweep_run
  *                                    then take this kernel for a table whose largest mesh is beyond the resident
- *                                    kernel's limit, and the resident kernels otherwise (the loss form
- *                                    p6d_add_forward and p6d_add_backward keep their limit). */
+ *                                    kernel's limit, and the resident kernels otherwise (evaluation only: the loss
+ *                                    form p6d_add_forward and p6d_add_backward follow
+ *                                    p6d_mesh_table_set_large_mesh_loss, below). */
 int p6d_mesh_table_set_large_meshes(p6d_mesh_table* table, int enable);
 int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                           const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
@@ -204,6 +205,33 @@ int p6d_add_forward(const p6d_mesh_table* table, const float* pq, const float* p
 int p6d_add_backward(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                      const float* gt, const int64_t* obj, int64_t B, const float* grad_out,
                      const int32_t* count, float inv_count, float* grad_q, float* grad_t, void* stream);
+
+/* OPT-IN: ADDLoss.forward and its gradient for meshes larger than shared memory.  p6d_add_forward refuses a table
+ * whose largest mesh is beyond p6d_adds_max_points (its resident ADD-S kernel), and p6d_add_backward one beyond
+ * ~19,000 points (it holds the gt cloud in shared memory), both with P6D_ETOOBIG.  The streamed loss form runs the
+ * streamed evaluation kernel with the batched matmul's rounding, scans the gt tiles for symmetric samples only and
+ * folds the per-sample values into the loss in a single-CTA launch after the last chunk: the same loss and count
+ * bits as p6d_add_forward wherever both run.  The streamed backward splits every pose into blocks of pred points,
+ * streams the gt cloud in 1,024-point tiles for symmetric samples with the resident kernel's nearest-point rule
+ * (first index of the smallest rooted distance, the first NaN wins, G = 0 where the distance is 0) carried across
+ * tiles, and sums the blocks' float64 partials in block order, so its result does not depend on scheduling.  Both
+ * allocate their per-point workspace stream-ordered on `stream` (at most 64 MB; larger batches run in chunks); the
+ * caller's workspace of p6d_add_forward_workspace_bytes is unchanged.  Tables above 32,768 points answer
+ * P6D_ETOOBIG with the reason of p6d_add_eval_streamed.
+ *   p6d_add_forward_streamed, p6d_add_backward_streamed
+ *                                        always the streamed kernels, for any mesh of 1 to 32,768 points; same
+ *                                        arguments as p6d_add_forward / p6d_add_backward
+ *   p6d_mesh_table_set_large_mesh_loss   per-table switch (default off): p6d_add_forward and p6d_add_backward then
+ *                                        take the streamed kernel for a table beyond their resident kernel's limit,
+ *                                        and the resident kernels (same kernel, same bytes as with the switch off)
+ *                                        otherwise.  Independent of p6d_mesh_table_set_large_meshes. */
+int p6d_mesh_table_set_large_mesh_loss(p6d_mesh_table* table, int enable);
+int p6d_add_forward_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                             const float* gt, const int64_t* obj, int64_t B, float* loss, int32_t* count,
+                             void* workspace, void* stream);
+int p6d_add_backward_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                              const float* gt, const int64_t* obj, int64_t B, const float* grad_out,
+                              const int32_t* count, float inv_count, float* grad_q, float* grad_t, void* stream);
 
 /* Quaternion -> rotation matrix, ADDLoss._quat_to_mat (models/add_loss.py:203-215). */
 int p6d_quat_to_mat(const float* q, int64_t B, float* R, int device, void* stream);
