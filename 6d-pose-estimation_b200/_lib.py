@@ -34,6 +34,7 @@ EXPORTS = (
     "p6d_mesh_table_set_large_meshes", "p6d_add_eval_host",
     "p6d_add_forward_workspace_bytes", "p6d_add_forward", "p6d_add_backward",
     "p6d_mesh_table_set_large_mesh_loss", "p6d_add_forward_streamed", "p6d_add_backward_streamed",
+    "p6d_mesh_table_set_large_mesh_pruning", "p6d_add_eval_pruned_streamed",
     "p6d_quat_to_mat", "p6d_pose_loss_workspace_bytes", "p6d_pose_loss_fwd_bwd",
     "p6d_pose_loss_pinhole_fwd_bwd", "p6d_pinhole_fwd", "p6d_pinhole_bwd", "p6d_depth_backproject",
     "p6d_depth_crop_backproject", "p6d_detection_backproject", "p6d_project_points", "p6d_synth_poses", "p6d_sweep_run",
@@ -89,6 +90,8 @@ def lib() -> C.CDLL:
     L.p6d_mesh_table_set_pruning.argtypes = [vp, i32]
     L.p6d_add_eval_streamed.argtypes = L.p6d_add_eval.argtypes
     L.p6d_mesh_table_set_large_meshes.argtypes = [vp, i32]
+    L.p6d_add_eval_pruned_streamed.argtypes = L.p6d_add_eval.argtypes
+    L.p6d_mesh_table_set_large_mesh_pruning.argtypes = [vp, i32]
     L.p6d_add_eval_host.argtypes = [vp, vp, vp, vp, vp, vp, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp,
                                     C.POINTER(i32)]
     L.p6d_add_forward_workspace_bytes.argtypes = [vp, i64]
@@ -248,21 +251,34 @@ class MeshTable:
         check(lib().p6d_mesh_table_set_large_mesh_loss(self.handle, 1 if enable else 0))
         return self
 
+    def set_large_mesh_pruning(self, enable=True):
+        """Opt in to (or out of) the streamed exact-pruned ADD-S kernel for this table: same bits as the other
+        evaluation kernels, taken for ADD-S evaluation only when the largest mesh is beyond the pruned kernel's
+        shared-memory limit (up to 32,768 points); independent of the other switches; refused for a table
+        without a block structure; see include/p6d.h."""
+        check(lib().p6d_mesh_table_set_large_mesh_pruning(self.handle, 1 if enable else 0))
+        return self
+
     # -- device-buffer evaluation ---------------------------------------------------
-    def evaluate_packed(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False):
+    def evaluate_packed(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False,
+                        prune_streamed=False):
         """Launch the evaluation kernels on the current stream and return the ONE buffer behind the
         per-pose outputs: add f32 [B] | adds f32 [B] | hit u8 [B] | valid u8 [B] | borderline u8 [B]
         (adds is left unwritten when want_adds is False).  All inputs must already be contiguous CUDA
         tensors on this table's device.  No views are created: at the reference's batch sizes every
         torch op is 2-3 us of a ~100 us call.  prune / streamed: always the exact-pruned (ADD-S only) or the
-        streamed kernel (p6d_add_eval_pruned / p6d_add_eval_streamed) instead of the table's choice."""
+        streamed kernel (p6d_add_eval_pruned / p6d_add_eval_streamed) instead of the table's choice.
+        prune_streamed: always the streamed exact-pruned kernel (p6d_add_eval_pruned_streamed, ADD-S only); it
+        takes precedence over prune / streamed."""
         B = obj.shape[0]
         out = torch.empty(11 * B + 16, dtype=torch.uint8, device=self.device)
         base = out.data_ptr()
         acc_struct = None
         if acc is not None:
             acc_struct = Accumulators(*(ptr(a) for a in acc))
-        if streamed:
+        if prune_streamed and want_adds:
+            entry = lib().p6d_add_eval_pruned_streamed
+        elif streamed:
             entry = lib().p6d_add_eval_streamed
         else:
             entry = lib().p6d_add_eval_pruned if (prune and want_adds) else lib().p6d_add_eval
@@ -272,11 +288,12 @@ class MeshTable:
                     stream_ptr(self.device)))
         return out
 
-    def evaluate(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False):
+    def evaluate(self, pq, pt, gq, gt, obj, want_adds=True, order=None, acc=None, prune=False, streamed=False,
+                 prune_streamed=False):
         """evaluate_packed + views: returns (add, adds, hit, valid, packed) device tensors (adds is
         None when want_adds is False)."""
         B = obj.shape[0]
-        out = self.evaluate_packed(pq, pt, gq, gt, obj, want_adds, order, acc, prune, streamed)
+        out = self.evaluate_packed(pq, pt, gq, gt, obj, want_adds, order, acc, prune, streamed, prune_streamed)
         add = out[: 4 * B].view(torch.float32)
         adds = out[4 * B: 8 * B].view(torch.float32)
         return add, (adds if want_adds else None), out[8 * B: 9 * B], out[9 * B: 10 * B], out

@@ -520,6 +520,8 @@ constexpr int PR_MIN_POINTS = 128;
 //   * without ADD-S: the ADD-only kernel (a); beyond its shared memory, the streamed kernel if the table's large-mesh
 //     switch is on;
 //   * pruning switch on, a block structure, a largest mesh of >= PR_MIN_POINTS that fits: the pruned kernel;
+//   * large-mesh pruning switch on, a block structure and a largest mesh beyond the pruned kernel's shared memory:
+//     the streamed pruned kernel (it refuses more than 32,768 points);
 //   * large-mesh switch on and a mesh beyond the resident kernel's shared memory: the streamed kernel;
 //   * otherwise the resident ADD-S kernel.
 // Wherever two of these kernels can run a call, they give the same bytes.
@@ -547,13 +549,16 @@ int launch_eval(const p6d_mesh_table* t, const EvalArgs& args, bool want_adds, c
         const bool large = t->large_meshes.load(std::memory_order_relaxed);
         const bool prune = want_adds && t->pruned && t->pruning.load(std::memory_order_relaxed) &&
                            t->max_count >= PR_MIN_POINTS;
+        const bool prune_large = want_adds && t->pruned && t->large_mesh_pruning.load(std::memory_order_relaxed);
         int limit = 0;
-        if ((large || prune) && (rc = max_optin_smem(t->device, &limit))) return rc;
+        if ((large || prune || prune_large) && (rc = max_optin_smem(t->device, &limit))) return rc;
         if (!want_adds)
             rc = large && !add_only_fits(t, limit) ? launch_eval_streamed(t, args, false, st)
                                                    : launch_add_only(t, args, st);
         else if (prune && pruned_fits(t, limit))
             rc = launch_eval_pruned(t, args, st);
+        else if (prune_large && !pruned_fits(t, limit))
+            rc = launch_eval_pruned_streamed(t, args, st);
         else if (large && !resident_fits(t, limit))
             rc = launch_eval_streamed(t, args, true, st);
         else if ((rc = pick_variant(t, false, st, &vi)) == P6D_OK)
@@ -819,21 +824,35 @@ int p6d_mesh_table_set_large_mesh_loss(p6d_mesh_table* table, int enable) {
     return P6D_OK;
 }
 
+int p6d_mesh_table_set_large_mesh_pruning(p6d_mesh_table* table, int enable) {
+    if (!table) { set_error("p6d_mesh_table_set_large_mesh_pruning: table is NULL"); return P6D_EINVAL; }
+    if (!table->pruned) {
+        if (!enable) return P6D_OK;
+        set_error("p6d_mesh_table_set_large_mesh_pruning: this table has no block structure (a mesh with more than "
+                  "65,534 points, or out of memory at creation)");
+        return P6D_ETOOBIG;
+    }
+    table->large_mesh_pruning.store(enable != 0, std::memory_order_relaxed);
+    return P6D_OK;
+}
+
 }  // extern "C"
 
 // float4 / float2 / int4 loads in the kernels need their natural alignment
 static bool misaligned(const void* p, size_t a) { return p && (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; }
 
-// The three device-buffer evaluation entries: p6d_add_eval routes through launch_eval, the other two launch their
+// The four device-buffer evaluation entries: p6d_add_eval routes through launch_eval, the other three launch their
 // kernel directly.  Error messages are prefixed with the entry's name.
-enum EvalEntry { EVAL_ROUTED, EVAL_PRUNED, EVAL_STREAMED };
+enum EvalEntry { EVAL_ROUTED, EVAL_PRUNED, EVAL_STREAMED, EVAL_PRUNED_STREAMED };
 
 static int eval_entry(EvalEntry which, const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
                       const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add, float* adds,
                       uint8_t* hit, uint8_t* valid, uint8_t* borderline, const p6d_accumulators* acc, void* stream) {
-    static const char* const names[] = {"p6d_add_eval", "p6d_add_eval_pruned", "p6d_add_eval_streamed"};
+    static const char* const names[] = {"p6d_add_eval", "p6d_add_eval_pruned", "p6d_add_eval_streamed",
+                                        "p6d_add_eval_pruned_streamed"};
     const char* fn = names[which];
-    const bool need_adds = which == EVAL_PRUNED;   // the pruned kernel computes ADD-S in any case
+    // the pruned kernels compute ADD-S in any case
+    const bool need_adds = which == EVAL_PRUNED || which == EVAL_PRUNED_STREAMED;
     if (!table || B < 0 || (B > 0 && (!pq || !pt || !gq || !gt || !obj || !add || (need_adds && !adds) || !hit || !valid))) {
         set_error("%s: bad arguments", fn);
         return P6D_EINVAL;
@@ -860,6 +879,7 @@ static int eval_entry(EvalEntry which, const p6d_mesh_table* table, const float*
     switch (which) {
         case EVAL_PRUNED: return launch_eval_pruned(table, a, st);
         case EVAL_STREAMED: return launch_eval_streamed(table, a, adds != nullptr, st);
+        case EVAL_PRUNED_STREAMED: return launch_eval_pruned_streamed(table, a, st);
         default: return launch_eval(table, a, adds != nullptr, st, nullptr);
     }
 }
@@ -886,6 +906,14 @@ int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const fl
                           const p6d_accumulators* acc, void* stream) {
     return eval_entry(EVAL_STREAMED, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid, borderline, acc,
                       stream);
+}
+
+int p6d_add_eval_pruned_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                                 const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
+                                 float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                                 const p6d_accumulators* acc, void* stream) {
+    return eval_entry(EVAL_PRUNED_STREAMED, table, pq, pt, gq, gt, obj, order, B, add, adds, hit, valid, borderline,
+                      acc, stream);
 }
 
 int64_t p6d_add_forward_workspace_bytes(const p6d_mesh_table* table, int64_t B) {

@@ -59,7 +59,14 @@ struct PrunedTable {
     std::vector<PrunedSlot> h_slots;
     int max_nb = 0;
     int max_count = 0;
+    // kernel (b''') only: model-space centroid of every super-block (PR_SUPER consecutive blocks) as float4, and the
+    // index of each object's first super-block in that array.  Kept apart from the block layout above, which kernel
+    // (b') stages in shared memory.
+    float4* d_super = nullptr;
+    int32_t* d_super_off = nullptr;
 };
+
+constexpr int PR_SUPER = 32;              // blocks per super-block of kernel (b'''): 1,024 points
 
 // k-d median splits: idx[lo, hi) -> blocks of 32 consecutive entries made of sub-blocks of 8, each spatially compact
 static void kd_split(const float* xyz, std::vector<int>& idx, int lo, int hi) {
@@ -101,6 +108,13 @@ static PrunedTable* build_blocks(const p6d_mesh_table* t, const float* xyz, cons
         pt->max_count = std::max(pt->max_count, n);
     }
     std::vector<float> buf(total > 0 ? total : 4, 0.0f);
+    std::vector<int32_t> super_off(t->n_slots);
+    int32_t n_super = 0;
+    for (int s = 0; s < t->n_slots; ++s) {
+        super_off[s] = n_super;
+        n_super += (pt->h_slots[s].nb + PR_SUPER - 1) / PR_SUPER;
+    }
+    std::vector<float4> super(n_super > 0 ? n_super : 1, make_float4(0.0f, 0.0f, 0.0f, 0.0f));
     for (int s = 0; s < t->n_slots; ++s) {
         const int n = t->h_slots[s].count;
         if (n == 0) continue;
@@ -138,15 +152,32 @@ static PrunedTable* build_blocks(const p6d_mesh_table* t, const float* xyz, cons
                     sub[k * ns + 4 * b + q] = scnt > 0 ? static_cast<float>(sc[k] / scnt) : x[k * np + PR_BLOCK * b];
             }
         }
+        // super-blocks: the sorted positions below n are exactly the mesh's points (only the last block is padded)
+        for (int S = 0; S * PR_SUPER < ps.nb; ++S) {
+            double c[3] = {0.0, 0.0, 0.0};
+            const int first = PR_SUPER * PR_BLOCK * S, last = std::min(n, first + PR_SUPER * PR_BLOCK);
+            for (int p = first; p < last; ++p)
+                for (int k = 0; k < 3; ++k) c[k] += x[k * np + p];
+            const double cnt = last - first;
+            super[super_off[s] + S] = make_float4(static_cast<float>(c[0] / cnt), static_cast<float>(c[1] / cnt),
+                                                  static_cast<float>(c[2] / cnt), 0.0f);
+        }
     }
     if (cudaMalloc(&pt->d_sorted, buf.size() * sizeof(float)) != cudaSuccess ||
         cudaMalloc(&pt->d_slots, t->n_slots * sizeof(PrunedSlot)) != cudaSuccess ||
+        cudaMalloc(&pt->d_super, super.size() * sizeof(float4)) != cudaSuccess ||
+        cudaMalloc(&pt->d_super_off, t->n_slots * sizeof(int32_t)) != cudaSuccess ||
         cudaMemcpy(pt->d_sorted, buf.data(), buf.size() * sizeof(float), cudaMemcpyHostToDevice) != cudaSuccess ||
         cudaMemcpy(pt->d_slots, pt->h_slots.data(), t->n_slots * sizeof(PrunedSlot), cudaMemcpyHostToDevice) !=
+            cudaSuccess ||
+        cudaMemcpy(pt->d_super, super.data(), super.size() * sizeof(float4), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemcpy(pt->d_super_off, super_off.data(), t->n_slots * sizeof(int32_t), cudaMemcpyHostToDevice) !=
             cudaSuccess) {
         cudaGetLastError();
         if (pt->d_sorted) cudaFree(pt->d_sorted);
         if (pt->d_slots) cudaFree(pt->d_slots);
+        if (pt->d_super) cudaFree(pt->d_super);
+        if (pt->d_super_off) cudaFree(pt->d_super_off);
         return nullptr;
     }
     return pt.release();
@@ -167,6 +198,8 @@ void free_pruned(PrunedTable* pt) {
     if (!pt) return;
     cudaFree(pt->d_sorted);
     cudaFree(pt->d_slots);
+    cudaFree(pt->d_super);
+    cudaFree(pt->d_super_off);
     delete pt;
 }
 
@@ -446,6 +479,353 @@ int launch_eval_pruned(const p6d_mesh_table* table, const EvalArgs& args, cudaSt
     P6D_CUDA(cudaLaunchKernel(pick->fn, dim3(static_cast<unsigned>(grid)), dim3(pick->threads), kargs, smem, st));
     P6D_CUDA(cudaGetLastError());
     return P6D_OK;
+}
+
+// ================================================================================================================
+// Kernel (b'''): exact block pruning for meshes beyond kernel (b')'s shared memory (opt-in), up to 32,768 points.
+//
+// Kernel (b') keeps the sorted mesh and both clouds in shared memory (~4,700 points).  This one keeps the per-pose
+// state in a workspace in global memory (the gt cloud of one pose is <= 384 KB and stays in L2) and splits every
+// pose into work items, in two launches per chunk of poses:
+//   pass 1  one CTA per (pose, super-block of PR_SUPER blocks): every warp runs phase B' of kernel (b') on its blocks
+//           -- the very xform_point calls, so the same coordinates, bit for bit -- and writes the ADD distance at the
+//           ORIGINAL index, the gt cloud in b''s quad layout (padded with GT_SENTINEL), the pred block spheres and
+//           the gt sub-block spheres; the CTA adds one gt sphere per super-block (centre = its transformed
+//           model-space centroid, radius = the bit-pattern maximum over its actual transformed points x 1.00001);
+//   pass 2  items of (pose, group of pred blocks) claimed by a persistent grid through an atomic counter, pred blocks
+//           claimed warp by warp inside the item as in phase C': one pred point per lane (re-transformed: the same
+//           bits as pass 1's), the same-index gt block first, then the gt SUPER-block spheres (one per lane) and
+//           only inside a surviving super-block its sub-block spheres, 32 per chunk; the survivors are evaluated
+//           with eval_sub / eval_two from the workspace.  A super-block is re-tested with the current minima before
+//           each descent.  The row minima go, __fsqrt_rn-ed, to the ADD-S row at the original index;
+//   finish  the last item of a pose (per-pose ticket after __threadfence, as in kernel (b'')) takes the ordered means
+//           from the workspace rows (__ldcg) and writes the outputs (write_pose); unknown ids go through
+//           write_skipped in the pose's first item.
+// A super-block or a sub-block is skipped only when  d^2 * 0.9999 >= (sqrt(max m) * 1.0001 + rA + rB)^2  holds in
+// numbers (the test of kernel (b')); a skipped super-block holds only sub-blocks that the same test at the same m
+// would skip, and m only decreases, so every minimum is the all-pairs minimum.  NaN and inf fail the test and are
+// evaluated.  With one level only, every pred block would test all 4 nb sub-blocks (4.2 M sphere tests per pose at
+// 32,768 points), as much as the pair work pruning leaves for a good prediction.
+// Workspace per pose (floats): ADD row, ADD-S row [stride each] | gt quads [3 * 32 nb] | pred spheres [nb] | gt
+// sub-block spheres [4 nb] | gt super-block spheres [nsb] (float4 each): about 22.5 bytes per point, allocated
+// stream-ordered on the caller's stream and kept within 64 MB by launching in chunks of poses.
+constexpr int PS_T = 256;                                 // threads per CTA, both passes
+constexpr int PS_WARPS = PS_T / 32;
+constexpr size_t PS_WS_BYTES = size_t(64) << 20;
+
+struct PsTable {
+    const float* sorted;
+    const PrunedSlot* pslots;
+    const float4* super;
+    const int32_t* super_off;
+};
+
+struct PsArgs {
+    int64_t first;      // first pose of the chunk in processing order
+    int nposes;         // poses in the chunk
+    int nsb;            // super-blocks of the table's largest mesh (pass 1: CTAs per pose)
+    int group;          // pred blocks per pass-2 item
+    int ipp;            // pass-2 items per pose of the table's largest mesh
+    int stride;         // floats per per-point row
+    int nb;             // blocks of the table's largest mesh
+    int pose_floats;    // floats of one pose's workspace
+    int* counter;       // pass-2 work counter (zeroed before the chunk)
+    int* tickets;       // [nposes] finished pass-2 items per pose (zeroed before the chunk)
+    float* ws;          // [nposes][pose_floats]
+};
+
+struct PsPose {         // one pose's workspace
+    float* row_add;
+    float* row_adds;
+    float* gq;
+    float4* cp;
+    float4* cg;
+    float4* cs;
+};
+
+__device__ __forceinline__ PsPose ps_pose(const PsArgs& sa, int pi) {
+    PsPose w;
+    w.row_add = sa.ws + static_cast<size_t>(pi) * sa.pose_floats;
+    w.row_adds = w.row_add + sa.stride;
+    w.gq = w.row_adds + sa.stride;
+    w.cp = reinterpret_cast<float4*>(w.gq + 3 * PR_BLOCK * sa.nb);
+    w.cg = w.cp + sa.nb;
+    w.cs = w.cg + 4 * sa.nb;
+    return w;
+}
+
+// kernel (b')'s test: the sphere B lies beyond th = sqrt(max m) * 1.0001 + rA of centre cA; false for NaN / inf
+__device__ __forceinline__ bool sphere_skips(const float4& cA, float th, const float4& cB) {
+    const float dx = cA.x - cB.x, dy = cA.y - cB.y, dz = cA.z - cB.z;
+    const float d2 = dx * dx + dy * dy + dz * dz;
+    const float rhs = th + cB.w;
+    return d2 * 0.9999f >= rhs * rhs && d2 < 3.0e38f;
+}
+
+template <int T>
+__global__ void __launch_bounds__(T) adds_pruned_streamed_xform_kernel(EvalArgs a, PsTable pa, PsArgs sa) {
+    constexpr int W = T / 32;
+    __shared__ float s_pose[14];
+    __shared__ long long s_oid;
+    __shared__ unsigned s_rs[W];
+    const unsigned full = 0xffffffffu;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int pi = static_cast<int>(blockIdx.x / sa.nsb), S = static_cast<int>(blockIdx.x % sa.nsb);
+    const int64_t idx = sa.first + pi;
+    const int64_t b = a.order ? a.order[idx] : idx;
+    load_pose(a, b, tid, s_pose, &s_oid);
+    __syncthreads();
+    const long long oid = s_oid;
+    if (!slot_known(oid, a.n_slots, a.slots)) return;     // CTA-uniform; pass 2 writes the outputs
+    const SlotInfo s = a.slots[oid];
+    const PrunedSlot ps = pa.pslots[oid];
+    const int nb = ps.nb, np = PR_BLOCK * nb, nbp = (nb + 3) / 4 * 4, ns = 4 * nb;
+    if (S * PR_SUPER >= nb) return;                        // beyond this pose's mesh
+    const float* mx = pa.sorted + ps.offset;
+    const float* my = mx + np;
+    const float* mz = my + np;
+    const float* cen = mz + np;
+    const float* sub = cen + 3 * nbp;
+    const uint16_t* perm = reinterpret_cast<const uint16_t*>(sub + 3 * ns);
+    const int mode = s.xform_mode;
+    const PsPose w = ps_pose(sa, pi);
+
+    float Rp[9], Rg[9], tp[3], tg[3];
+    quat_to_mat(s_pose, Rp);
+    quat_to_mat(s_pose + 4, Rg);
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        tp[k] = s_pose[8 + k];
+        tg[k] = s_pose[11 + k];
+    }
+    const float4 cS = pa.super[pa.super_off[oid] + S];
+    float csx, csy, csz;
+    xform_point(XF_FMA_CHAIN, cS.x, cS.y, cS.z, Rg, tg, csx, csy, csz);
+    unsigned rs = 0u;
+    const int blk_end = min(nb, PR_SUPER * (S + 1));
+    for (int blk = PR_SUPER * S + warp; blk < blk_end; blk += W) {
+        // phase B' of kernel (b'), into the workspace
+        const int p = PR_BLOCK * blk + lane;
+        const unsigned orig = perm[p];
+        const bool valid = orig != 0xffffu;
+        const float x = mx[p], y = my[p], z = mz[p];
+        float px, py, pz, qx, qy, qz;
+        xform_point(mode, x, y, z, Rp, tp, px, py, pz);
+        xform_point(mode, x, y, z, Rg, tg, qx, qy, qz);
+        float* gq = w.gq + (p >> 2) * 12 + (p & 3);
+        gq[0] = valid ? qx : GT_SENTINEL;
+        gq[4] = valid ? qy : GT_SENTINEL;
+        gq[8] = valid ? qz : GT_SENTINEL;
+        if (valid) w.row_add[orig] = __fsqrt_rn(sq3(__fsub_rn(px, qx), __fsub_rn(py, qy), __fsub_rn(pz, qz)));
+        const float cx = cen[blk], cy = cen[nbp + blk], cz = cen[2 * nbp + blk];
+        const int sb = 4 * blk + (lane >> 3);
+        const float sx = sub[sb], sy = sub[ns + sb], sz = sub[2 * ns + sb];
+        float cpx, cpy, cpz, cgx, cgy, cgz;
+        xform_point(XF_FMA_CHAIN, cx, cy, cz, Rp, tp, cpx, cpy, cpz);
+        xform_point(XF_FMA_CHAIN, sx, sy, sz, Rg, tg, cgx, cgy, cgz);
+        const float dp = sqrtf(sq3(px - cpx, py - cpy, pz - cpz));
+        const float dg = sqrtf(sq3(qx - cgx, qy - cgy, qz - cgz));
+        const float ds = sqrtf(sq3(qx - csx, qy - csy, qz - csz));
+        const unsigned rp = __reduce_max_sync(full, valid ? __float_as_uint(dp) : 0u);
+        unsigned rg = valid ? __float_as_uint(dg) : 0u;
+        rg = max(rg, __shfl_xor_sync(full, rg, 1));
+        rg = max(rg, __shfl_xor_sync(full, rg, 2));
+        rg = max(rg, __shfl_xor_sync(full, rg, 4));
+        rs = max(rs, valid ? __float_as_uint(ds) : 0u);
+        if (lane == 0) w.cp[blk] = make_float4(cpx, cpy, cpz, __uint_as_float(rp) * 1.00001f);
+        if ((lane & 7) == 0) w.cg[sb] = make_float4(cgx, cgy, cgz, __uint_as_float(rg) * 1.00001f);
+    }
+    rs = __reduce_max_sync(full, rs);
+    if (lane == 0) s_rs[warp] = rs;
+    __syncthreads();
+    if (tid == 0) {
+        unsigned r = s_rs[0];
+#pragma unroll
+        for (int k = 1; k < W; ++k) r = max(r, s_rs[k]);
+        w.cs[S] = make_float4(csx, csy, csz, __uint_as_float(r) * 1.00001f);
+    }
+}
+
+template <int T, int MINB>
+__global__ void __launch_bounds__(T, MINB) adds_pruned_streamed_kernel(EvalArgs a, PsTable pa, PsArgs sa) {
+    constexpr int W = T / 32;
+    __shared__ float s_pose[14];
+    __shared__ float s_mean[2];
+    __shared__ long long s_oid;
+    __shared__ int s_item, s_last, s_blk;
+    const unsigned full = 0xffffffffu;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int64_t total = static_cast<int64_t>(sa.nposes) * sa.ipp;
+
+    for (;;) {
+        if (tid == 0) {
+            s_item = atomicAdd(sa.counter, 1);
+            s_blk = W;               // nobody reads it between the previous item's last barrier and (B)
+        }
+        __syncthreads();  // (A) also: the previous item is done with s_pose
+        const int64_t it = s_item;
+        if (it >= total) break;
+        const int pi = static_cast<int>(it / sa.ipp), j = static_cast<int>(it % sa.ipp);
+        const int64_t idx = sa.first + pi;
+        const int64_t b = a.order ? a.order[idx] : idx;
+        load_pose(a, b, tid, s_pose, &s_oid);
+        __syncthreads();  // (B) also: every thread has read s_item
+        const long long oid = s_oid;
+        if (!slot_known(oid, a.n_slots, a.slots)) {   // CTA-uniform; the first item of the pose writes its outputs
+            if (tid == 0 && j == 0) write_skipped(a, b, true);
+            continue;
+        }
+        const PrunedSlot ps = pa.pslots[oid];
+        const int nb = ps.nb, np = PR_BLOCK * nb, ns = 4 * nb;
+        const int A0 = j * sa.group;
+        if (A0 >= nb) continue;    // beyond this pose's mesh: not counted in its ticket
+        const int A1 = min(nb, A0 + sa.group), items = (nb + sa.group - 1) / sa.group;
+        const int nsb = (nb + PR_SUPER - 1) / PR_SUPER;     // <= 32: one super-block per lane
+        const float* mx = pa.sorted + ps.offset;
+        const float* my = mx + np;
+        const float* mz = my + np;
+        const uint16_t* perm =
+            reinterpret_cast<const uint16_t*>(mz + np + 3 * ((nb + 3) / 4 * 4) + 3 * ns);
+        const int mode = a.slots[oid].xform_mode;
+        const PsPose w = ps_pose(sa, pi);
+        const float4* gq4 = reinterpret_cast<const float4*>(w.gq);   // block B at gq4[24 B ..], sub-block at gq4[6 SB ..]
+
+        float Rp[9], tp[3];
+        quat_to_mat(s_pose, Rp);
+#pragma unroll
+        for (int k = 0; k < 3; ++k) tp[k] = s_pose[8 + k];
+        int A = A0 + warp;
+        while (A < A1) {
+            const int p = PR_BLOCK * A + lane;
+            const unsigned orig = perm[p];
+            const bool valid = orig != 0xffffu;
+            float px, py, pz;
+            xform_point(mode, mx[p], my[p], mz[p], Rp, tp, px, py, pz);
+            // the same-index block as two trips of two sub-blocks (min is exact, so the grouping changes no bit):
+            // eval_block's 24 global loads at once would need more registers than three CTAs per SM leave
+            float m = __int_as_float(0x7f800000);
+#pragma unroll 1
+            for (int q = 0; q < 4; q += 2) m = eval_two(gq4 + 24 * A + 6 * q, gq4 + 24 * A + 6 * q + 6, px, py, pz, m);
+            const float4 cA = w.cp[A];
+            const float4 cS = lane < nsb ? w.cs[lane] : make_float4(0.0f, 0.0f, 0.0f, 0.0f);
+            unsigned left = nsb == 32 ? full : (1u << nsb) - 1u;   // super-blocks not yet evaluated or skipped
+            for (;;) {
+                // the bound uses the current minima: re-tested before every descent
+                float mmax = __uint_as_float(__reduce_max_sync(full, valid ? __float_as_uint(m) : 0u));
+                float th = sqrtf(mmax) * 1.0001f + cA.w;
+                const bool candS = ((left >> lane) & 1u) && !sphere_skips(cA, th, cS);
+                const unsigned todoS = __ballot_sync(full, candS);
+                if (!todoS) break;
+                const int S = __ffs(todoS) - 1;
+                left = todoS & ~(1u << S);     // a skipped super-block stays skipped: m only decreases
+                const int q1 = min(ns, 4 * PR_SUPER * (S + 1));
+                for (int c0 = 4 * PR_SUPER * S; c0 < q1; c0 += 32) {
+                    mmax = __uint_as_float(__reduce_max_sync(full, valid ? __float_as_uint(m) : 0u));
+                    th = sqrtf(mmax) * 1.0001f + cA.w;
+                    const int Bq = c0 + lane;
+                    const bool cand = Bq < q1 && (Bq >> 2) != A && !sphere_skips(cA, th, w.cg[Bq]);
+                    unsigned todo = __ballot_sync(full, cand);
+                    while (todo) {
+                        const int b0 = __ffs(todo) - 1;
+                        todo &= todo - 1;
+                        if (todo) {
+                            const int b1 = __ffs(todo) - 1;
+                            todo &= todo - 1;
+                            m = eval_two(gq4 + 6 * (c0 + b0), gq4 + 6 * (c0 + b1), px, py, pz, m);
+                        } else {
+                            m = eval_sub(gq4 + 6 * (c0 + b0), px, py, pz, m);
+                        }
+                    }
+                }
+            }
+            // sqrt is monotone and correctly rounded: sqrt(min s) == min sqrt(s)
+            if (valid) w.row_adds[orig] = __fsqrt_rn(m);
+            int nxt = 0;
+            if (lane == 0) nxt = A0 + atomicAdd(&s_blk, 1);
+            A = __shfl_sync(full, nxt, 0);
+        }
+
+        // the last item of the pose to finish computes the means
+        __threadfence();
+        __syncthreads();
+        if (tid == 0) s_last = atomicAdd(sa.tickets + pi, 1) == items - 1;
+        __syncthreads();
+        if (!s_last) continue;
+        __threadfence();
+        if (tid < 64) {
+            const SlotInfo s = a.slots[oid];     // read here: not held in registers across the scan
+            ordered_means(w.row_add, w.row_adds, s.count, tid, lane, true, s_mean,
+                          [](const float* p) { return __ldcg(p); });
+            if (tid == 0) write_pose(a, b, oid, s, s_mean[0], s_mean[1], true);
+        }
+    }
+}
+
+// Kernel (b''') for one evaluation launch: any table with a block structure and a largest mesh of 1 to 32,768
+// points (launch_eval takes it beyond kernel (b')'s shared memory when the table's switch is on).
+int launch_eval_pruned_streamed(const p6d_mesh_table* t, const EvalArgs& args, cudaStream_t st) {
+    const PrunedTable* ptab = t->pruned;
+    if (!ptab) {
+        set_error("p6d_add_eval_pruned_streamed: this table has no block structure (a mesh with more than 65,534 "
+                  "points, or out of memory at creation)");
+        return P6D_ETOOBIG;
+    }
+    int rc = check_streamed_size(t);
+    if (rc) return rc;
+    if (args.B == 0) return P6D_OK;
+    const int nb = ptab->max_nb > 0 ? ptab->max_nb : 1;
+    const int nsb = (nb + PR_SUPER - 1) / PR_SUPER;
+    const int nmax = t->max_count > 0 ? t->max_count : 1;
+    const int stride = (nmax + 3) / 4 * 4;
+    const int pose_floats = 2 * stride + 3 * PR_BLOCK * nb + 4 * nb + 16 * nb + 4 * nsb;
+    const size_t per_pose = sizeof(float) * static_cast<size_t>(pose_floats) + sizeof(int);
+    const int64_t bc = std::max<int64_t>(1, std::min<int64_t>(args.B, static_cast<int64_t>(PS_WS_BYTES / per_pose)));
+    const size_t head = 16 + (sizeof(int) * static_cast<size_t>(bc) + 15) / 16 * 16;
+    const size_t ws_bytes = head + sizeof(float) * static_cast<size_t>(pose_floats) * static_cast<size_t>(bc);
+
+    const void* scan = (const void*)adds_pruned_streamed_kernel<PS_T, 3>;
+    const void* xform = (const void*)adds_pruned_streamed_xform_kernel<PS_T>;
+    int per_sm = 0;
+    if ((rc = ctas_per_sm(scan, PS_T, t->device, 0, &per_sm))) return rc;
+    // the largest group of pred blocks per item whose items fill the device at least twice; 8 blocks otherwise
+    const int64_t slots = static_cast<int64_t>(t->sm_count) * per_sm;
+    int group = 8;
+    for (int g = PR_SUPER; g > 8; g /= 2)
+        if (bc * ((nb + g - 1) / g) >= 2 * slots) { group = g; break; }
+    const int ipp = (nb + group - 1) / group;
+
+    char* ws = nullptr;
+    P6D_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&ws), ws_bytes, st));
+    for (int64_t c0 = 0; c0 < args.B && rc == P6D_OK; c0 += bc) {
+        const int64_t nc = std::min<int64_t>(bc, args.B - c0);
+        PsArgs sa;
+        sa.first = c0;
+        sa.nposes = static_cast<int>(nc);
+        sa.nsb = nsb;
+        sa.group = group;
+        sa.ipp = ipp;
+        sa.stride = stride;
+        sa.nb = nb;
+        sa.pose_floats = pose_floats;
+        sa.counter = reinterpret_cast<int*>(ws);
+        sa.tickets = reinterpret_cast<int*>(ws + 16);
+        sa.ws = reinterpret_cast<float*>(ws + head);
+        PsTable pa{ptab->d_sorted, ptab->d_slots, ptab->d_super, ptab->d_super_off};
+        EvalArgs a = args;
+        void* kargs[] = {&a, &pa, &sa};
+        cudaError_t e = cudaMemsetAsync(ws, 0, 16 + sizeof(int) * static_cast<size_t>(nc), st);
+        if (e != cudaSuccess) { rc = cuda_fail(e, "cudaMemsetAsync(pruned streamed workspace)"); break; }
+        e = cudaLaunchKernel(xform, dim3(static_cast<unsigned>(nc * nsb)), dim3(PS_T), kargs, 0, st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) { rc = cuda_fail(e, "cudaLaunchKernel(adds_pruned_streamed_xform_kernel)"); break; }
+        const int64_t grid = std::min<int64_t>(nc * ipp, slots);
+        e = cudaLaunchKernel(scan, dim3(static_cast<unsigned>(grid)), dim3(PS_T), kargs, 0, st);
+        if (e == cudaSuccess) e = cudaGetLastError();
+        if (e != cudaSuccess) rc = cuda_fail(e, "cudaLaunchKernel(adds_pruned_streamed_kernel)");
+    }
+    const cudaError_t ef = cudaFreeAsync(ws, st);
+    if (rc == P6D_OK && ef != cudaSuccess) rc = cuda_fail(ef, "cudaFreeAsync(pruned streamed workspace)");
+    return rc;
 }
 
 }  // namespace p6d

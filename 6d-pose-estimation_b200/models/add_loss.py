@@ -78,6 +78,7 @@ class ADDLoss(nn.Module):
         self._table_pruning = False
         self._table_large = False
         self._table_large_loss = False
+        self._table_large_pruning = False
         # optional callable(indices, pred_r, pred_t, gt_r, gt_t, obj_ids) -> 0/1 per index, consulted by
         # eval_metrics for decisions flagged `borderline`; None (default): the kernel's decision stands
         self.borderline_resolver = None
@@ -91,6 +92,9 @@ class ADDLoss(nn.Module):
         # kernels in forward / train_loss and loss.backward() (same loss bits; the resident kernels wherever they
         # run) -- not part of the reference surface, default off
         self.large_mesh_loss = False
+        # opt-in: exact block pruning for meshes beyond the pruned kernel's shared memory (up to 32,768 points) in
+        # eval_metrics / eval_poses (same bits; evaluation only) -- not part of the reference surface, default off
+        self.large_mesh_pruning = False
         self._load_models(model_dir)
 
     # ------------------------------------------------------------------ loading
@@ -155,6 +159,7 @@ class ADDLoss(nn.Module):
             self._table_pruning = False
             self._table_large = False
             self._table_large_loss = False
+            self._table_large_pruning = False
         if bool(self.exact_pruning) != self._table_pruning:
             self._table.set_pruning(bool(self.exact_pruning))
             self._table_pruning = bool(self.exact_pruning)
@@ -164,6 +169,9 @@ class ADDLoss(nn.Module):
         if bool(self.large_mesh_loss) != self._table_large_loss:
             self._table.set_large_mesh_loss(bool(self.large_mesh_loss))
             self._table_large_loss = bool(self.large_mesh_loss)
+        if bool(self.large_mesh_pruning) != self._table_large_pruning:
+            self._table.set_large_mesh_pruning(bool(self.large_mesh_pruning))
+            self._table_large_pruning = bool(self.large_mesh_pruning)
         return self._table
 
     def _prepare(self, pred_r, pred_t, gt_r, gt_t, obj_ids, sort=True):

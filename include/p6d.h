@@ -162,6 +162,32 @@ int p6d_add_eval_streamed(const p6d_mesh_table* table, const float* pq, const fl
                           float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
                           const p6d_accumulators* acc, void* stream);
 
+/* OPT-IN: exact block pruning (as p6d_add_eval_pruned) for meshes beyond that kernel's shared memory, up to 32,768
+ * points; the same outputs, bit for bit, as p6d_add_eval_streamed and, wherever they run, the resident kernels.  Per
+ * chunk of poses a first launch transforms the mesh block by block into a workspace in global memory (gt cloud,
+ * ADD distances, bounding spheres per pred block, per 8-point gt sub-block and per 1,024-point gt super-block); a
+ * second one evaluates every pred block against the same-index gt block and then against the sub-blocks of the
+ * super-blocks that the sphere test keeps.  Workspace: about 22.5 bytes per point and pose (at most 64 MB; larger
+ * batches run in chunks), stream-ordered on `stream`; no host synchronisation.  Above 32,768 points the call answers
+ * P6D_ETOOBIG with the reason of p6d_add_eval_streamed.
+ *   p6d_add_eval_pruned_streamed           always this kernel, for any mesh of 1 to 32,768 points of a table with a
+ *                                          block structure; adds must not be NULL
+ *   p6d_mesh_table_set_large_mesh_pruning  per-table switch (default off; refused, like p6d_mesh_table_set_pruning,
+ *                                          for a table without a block structure): p6d_add_eval, p6d_add_eval_host
+ *                                          and p6d_sweep_run then take this kernel for ADD-S calls on a table whose
+ *                                          largest mesh is beyond p6d_add_eval_pruned's shared memory (~4,700
+ *                                          points), and their other routes otherwise.  Independent of the other
+ *                                          switches; the loss form and the backward never take it.  Like
+ *                                          p6d_add_eval_pruned it pays most for good predictions: measured on a B200
+ *                                          (DESIGN.md §4 b''') 1.5-27x the rate of p6d_add_eval_streamed at sigma
+ *                                          <= 0.1 rad, but for 16-pose calls on an 8,192-point box mesh it is only
+ *                                          level at sigma 0.1 and 0.83x at sigma 0.5. */
+int p6d_mesh_table_set_large_mesh_pruning(p6d_mesh_table* table, int enable);
+int p6d_add_eval_pruned_streamed(const p6d_mesh_table* table, const float* pq, const float* pt, const float* gq,
+                                 const float* gt, const int64_t* obj, const int32_t* order, int64_t B, float* add,
+                                 float* adds, uint8_t* hit, uint8_t* valid, uint8_t* borderline,
+                                 const p6d_accumulators* acc, void* stream);
+
 /* Same computation with HOST buffers: stages inputs to the device, runs the kernels,
  * copies results back and synchronises (the end-to-end path of bench.py).  acc_* are
  * host arrays [n_slots] that receive (not accumulate) the per-object totals; nullable.
